@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Llama-3-8B Q4_K_M batch-1 decode on B200 through the ggml-b200 C ABI (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one decoded token: one pass of the whole hot path (32 layers of rms_norm -> Q4_K/Q6_K GEMV x7 -> rope ->
 KV store -> flash_attn_ext -> ..., then the 128256-row output GEMV) over a 512-token context.
@@ -179,6 +179,8 @@ def main():
     ap.add_argument("--no-batch", action="store_true", help="skip the bs32-decode / prefill legs")
     ap.add_argument("--tp-model", default="llama3-70b", help="N>1: model of the extra row-split tensor-parallel leg ('' = skip)")
     ap.add_argument("--tp-layers", type=int, default=0, help="debug: fewer layers in the TP leg (reported as INVALID)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the logits of the last timed step (rank 0) to DIR/logits.npy, "
+                    "float32 [1, n_vocab]; inputs and weights are seeded, so two builds can be compared output for output")
     a = ap.parse_args()
     if a.impl == "reference":
         return reference_arm(a)
@@ -246,6 +248,9 @@ def main():
     L.b200_event_synchronize(e1)
     barrier()
     ms = L.b200_event_elapsed_ms(e0, e1)
+    if a.dump_outputs and rank == 0:          # the later legs overwrite g.logits (the roofline leg skips attention)
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "logits.npy"), g.logits[:g.V].reshape(1, g.V).cpu().numpy())
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -3,7 +3,8 @@ stay on the device and match the reference CPU backend.
   * K-shift  -- llama_context::build_rope_shift / build_kv_self_shift (llama-context.cpp:464-588): f16 K is re-rotated IN PLACE by
                 ROPE on f16 with an I32 per-cell shift; quantised K goes CPY(q -> f32), ROPE(f32, in place), CPY(f32 -> q);
   * defrag   -- build_kv_self_defrag (llama-context.cpp:590-...): runs of cache rows moved by same-type CPY between 2-D views.
-The expected bytes come from the reference itself (the same graph on its CPU backend, tests/reflib.py ref_k_shift)."""
+The expected K-shift bytes are the same graph computed by the oracle, whose dequantisers, rope and quantisers are pinned bit for bit
+to the reference (tests/test_oracle_pin.py); where oracle/_ref is built they are also checked against the reference's CPU backend."""
 import numpy as np
 import pytest
 
@@ -32,6 +33,15 @@ def k_shift_ops(b200, kd, kt, shift_d, tmp_d):
     return [b200.make_op(b200.OP_CPY, tmp, [kview]), b200.make_op(b200.OP_ROPE, tmp, [tmp, sh, None], params), b200.make_op(b200.OP_CPY, kview, [tmp])]
 
 
+def oracle_k_shift(kbytes, kt, shift):
+    """build_rope_shift on the oracle: f16 K is widened, roped in f32 and rounded back (ggml-cpu rope_f16); quantised K goes
+    dequantise -> rope -> quantise (ggml_cast, ggml_rope_ext_inplace, ggml_cpy)"""
+    k = kbytes.view(np.float16).astype(np.float32) if kt == R.F16 else R.orc_dequantize(kt, kbytes, D)
+    k = R.orc_rope(k.reshape(CELLS, HKV, D), shift, ROPE["n_rot"], ROPE["mode"], ROPE["freq_base"], freq_scale=ROPE["freq_scale"],
+                   n_ctx_orig=ROPE["n_ctx_orig"])
+    return k.astype(np.float16).view(np.uint8).reshape(-1) if kt == R.F16 else quant_rows(kt, k).reshape(-1)
+
+
 @pytest.mark.parametrize("exact", [1, 0])
 @pytest.mark.parametrize("kt", [R.F16, R.Q8_0, R.Q4_0])
 def test_k_shift_graph_matches_reference(b200, ctx, kt, exact):
@@ -40,7 +50,9 @@ def test_k_shift_graph_matches_reference(b200, ctx, kt, exact):
     kb = k.astype(np.float16).view(np.uint8).reshape(-1) if kt == R.F16 else quant_rows(kt, k).reshape(-1)
     shift = rng.integers(-64, 65, CELLS).astype(np.int32)
     shift[::7] = 0
-    want = R.ref_k_shift(kb, kt, D, HKV, CELLS, shift, **ROPE)
+    want = oracle_k_shift(kb, kt, shift)
+    if R.have_ref():
+        assert np.array_equal(want, R.ref_k_shift(kb, kt, D, HKV, CELLS, shift, **ROPE))
     kd, sd, tmp = to_dev(kb), to_dev(shift), dev_bytes(CELLS * HKV * D * 4)
     ops = k_shift_ops(b200, kd, kt, sd, tmp)
     for o in ops:
@@ -53,7 +65,7 @@ def test_k_shift_graph_matches_reference(b200, ctx, kt, exact):
         ctx.set_option("cpu_exact", 0)
     got = kd.cpu().numpy()
     if exact:
-        assert np.array_equal(got, want), "cpu-exact mode: K-shift bytes must equal the reference CPU backend's"
+        assert np.array_equal(got, want), "cpu-exact mode: K-shift bytes must equal the reference CPU arithmetic's"
     else:
         # fast mode: CUDA sincosf instead of glibc's; a value may land one rounding step away
         if kt == R.F16:

@@ -80,8 +80,9 @@ def test_reference_own_quantize_tests_pass():
     assert p.returncode == 0, p.stdout[-2000:]
 
 
-# ----------------------------------------------------------------------------- glue ops + flash attention (tests/golden/ops_golden.npz)
-OPS = np.load(os.path.join(os.path.dirname(__file__), "golden", "ops_golden.npz"))
+# ----------------------------------------------------------------------------- glue ops + flash attention (tests/golden/ops_golden*.npz)
+OPS = dict(np.load(os.path.join(os.path.dirname(__file__), "golden", "ops_golden.npz")))
+OPS.update(np.load(os.path.join(os.path.dirname(__file__), "golden", "ops_golden_fa_long.npz")))
 
 
 def _close(got, want, tol):

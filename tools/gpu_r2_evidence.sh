@@ -1,6 +1,7 @@
 #!/bin/bash
 # round-2 evidence: int8 tensor peak, per-config numbers, ncu launch list of the bench step + full captures of the hot kernels
 mkdir -p gpurun_out
+nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o tools/micro/i8_peak.bin tools/micro/i8_peak.cu
 ./tools/micro/i8_peak.bin 2>&1 | tee gpurun_out/r2_i8_peak.txt
 timeout 1200 python tools/bench_configs.py > gpurun_out/r2_configs.jsonl 2> gpurun_out/r2_configs.err; cat gpurun_out/r2_configs.jsonl; tail -2 gpurun_out/r2_configs.err
 # launch list of the bench command (cold-cache, serialised: shares only)
