@@ -18,7 +18,6 @@ void b200_set_error(const char *fmt, ...) {
 }
 
 void graph_cache_free(b200_ctx *ctx);   // graph.cu
-void dstep_cache_free(b200_ctx *ctx);   // dstep.cu
 
 void *b200_ctx::get_scratch(int slot, size_t size) {
     if (size <= scratch_size[slot]) return scratch[slot];
@@ -30,7 +29,6 @@ void *b200_ctx::get_scratch(int slot, size_t size) {
     // reallocation would read and write freed memory.  Drop every captured graph (they are re-captured on the next
     // sightings); scratch growth is rare (sizes grow by 25% and the large areas are allocated at their upper bound).
     graph_cache_free(this);
-    scratch_gen++;
     if (scratch[slot]) cudaFree(scratch[slot]);
     scratch[slot] = nullptr; scratch_size[slot] = 0;
     void *p = nullptr;
@@ -47,7 +45,6 @@ void *b200_ctx::get_scratch(int slot, size_t size) {
 }
 
 struct b200_event { int device; cudaEvent_t ev; };
-extern int g_gemm_desc_swap;            // gemm_i8.cu
 
 extern "C" {
 
@@ -102,11 +99,9 @@ b200_ctx *b200_ctx_create(int device) {
     if (const char *e = getenv("GGML_B200_GRAPHS")) ctx->opt_cuda_graphs = atoi(e);
     if (const char *e = getenv("GGML_B200_FUSION")) ctx->opt_fusion = atoi(e);
     if (const char *e = getenv("GGML_B200_PDL")) ctx->opt_pdl = atoi(e);
-    if (const char *e = getenv("GGML_B200_FA_MERGE")) ctx->opt_fa_merge_in_wo = atoi(e);      // 1: the output projection's GEMV merges the flash-attention KV splits (opt-in, measured slower)
     if (const char *e = getenv("GGML_B200_FFN_PAIR")) ctx->opt_ffn_pair = atoi(e);
     if (const char *e = getenv("GGML_B200_FA_EXACT")) ctx->opt_cpu_exact = atoi(e);
     if (const char *e = getenv("GGML_B200_CPU_EXACT")) ctx->opt_cpu_exact = atoi(e);
-    if (const char *e = getenv("GGML_B200_DSTEP")) ctx->opt_dstep = atoi(e);
     return ctx;
 }
 
@@ -115,15 +110,12 @@ void b200_ctx_destroy(b200_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     graph_cache_free(ctx);
-    dstep_cache_free(ctx);
-    if (ctx->eager_kv_table) cudaFree(ctx->eager_kv_table);
     b200_comm_destroy(ctx);
     for (int i = 0; i < 16; i++) {
         if (ctx->split_join[i]) cudaEventDestroy(ctx->split_join[i]);
         if (ctx->split_peer[i]) { b200_ctx_destroy(ctx->split_peer[i]); cudaSetDevice(ctx->device); }
     }
     if (ctx->split_fork) cudaEventDestroy(ctx->split_fork);
-    if (ctx->fattn_counters) cudaFree(ctx->fattn_counters);
     for (int i = 0; i < SCRATCH_COUNT; i++) if (ctx->scratch[i]) cudaFree(ctx->scratch[i]);
     cudaStreamDestroy(ctx->stream);
     delete ctx;
@@ -142,8 +134,8 @@ int b200_synchronize(b200_ctx *ctx) {
 int b200_set_option(b200_ctx *ctx, const char *key, int value) {
     std::string k(key);
     int *slot = k == "fusion" ? &ctx->opt_fusion : k == "pdl" ? &ctx->opt_pdl : k == "l2_prefetch" ? &ctx->opt_l2_prefetch :
-                k == "debug_skip" ? &ctx->opt_debug_skip : (k == "fa_exact" || k == "cpu_exact") ? &ctx->opt_cpu_exact : k == "dstep" ? &ctx->opt_dstep :
-                k == "ffn_pair" ? &ctx->opt_ffn_pair : k == "fa_merge_in_wo" ? &ctx->opt_fa_merge_in_wo : nullptr;
+                k == "debug_skip" ? &ctx->opt_debug_skip : (k == "fa_exact" || k == "cpu_exact") ? &ctx->opt_cpu_exact :
+                k == "ffn_pair" ? &ctx->opt_ffn_pair : nullptr;
     if (k == "cuda_graphs") ctx->opt_cuda_graphs = value;
     else if (slot) {
         if (*slot != value) {                 // captured graphs bake these options in: drop them
@@ -153,7 +145,6 @@ int b200_set_option(b200_ctx *ctx, const char *key, int value) {
         }
         *slot = value;
     }
-    else if (k == "gemm_desc_swap") g_gemm_desc_swap = value;
     else { b200_set_error("unknown option %s", key); return B200_ERR_UNSUPPORTED; }
     return B200_OK;
 }

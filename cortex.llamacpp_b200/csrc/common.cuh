@@ -123,7 +123,6 @@ struct b200_ctx {
     void *        scratch[6]      = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     size_t        scratch_size[6] = {0, 0, 0, 0, 0, 0};
     int64_t       launches = 0;
-    int64_t       scratch_gen = 0;          // bumped on every scratch reallocation (captured graphs are dropped with it)
     // options
     int           opt_cuda_graphs = 0;
     int           opt_fusion      = 2;      // 0 off, 1 two-op fusions, 2 + llama layer fusions for decode ubatches
@@ -134,23 +133,11 @@ struct b200_ctx {
                                             // V accumulator of f16-cache attention, correctly rounded exp/sin/cos.  Slow; proves summation order is the only difference
     int           opt_debug_skip  = 0;      // timing experiments only: bit 0 flash_attn, 1 rope+store, 2 GEMV are not launched
     GraphCache *  graph_cache = nullptr;
-    void *        dstep_cache = nullptr;       // decode-step programs (dstep.cu)
-    void **       eager_kv_table = nullptr;    // KV-store destinations of eagerly run decode-step programs (graph.cu)
-    int           opt_dstep = 0;               // 1: a batch-1 decode step runs as ONE persistent kernel (dstep.cu).  Opt-in: correct, but measured
-                                               // slower than the per-launch path on B200 (2.66 vs 1.88 ms/step, profiles/r2_dstep_timeline.md)
     // live-tile map of the attention mask (fattn.cu): built by the first FLASH_ATTN_EXT of a graph that uses a given mask, reused by
     // the other layers; dropped at every graph_compute / compute_op entry and when an op writes into the mask
-    // decode fusion "split merge in the consumer": graph.cu asks the flash-attention launch to leave its KV-split partials unmerged
-    // (fa_skip_combine) when the batch-1 GEMV of the attention output projection will merge them in its activation prologue; the launch
-    // answers with where the partials are (fa_part_ns = 0: it merged them itself, dst is valid)
-    bool          fa_skip_combine = false;
-    const float * fa_part = nullptr;
-    int           fa_part_ns = 0, fa_part_gq = 0;
-    int           opt_fa_merge_in_wo = 0;       // measured slower (532 vs 555 tok/s): 148 CTAs re-reading the same ~100 KB of partials is an L2 hot spot (5 us); opt-in
     bool          fa_map_valid = false;
     uintptr_t     fa_map_mask = 0, fa_map_mask_end = 0;
     int64_t       fa_map_key[4] = {0, 0, 0, 0};        // m_nb1, n_kv, n_q, QC
-    void *        fattn_counters = nullptr;   // split-arrival counters of the fused flash-attention combine (fattn.cu)
     b200_comm *   comm = nullptr;       // tensor-parallel communicator (comm.cu); NULL = single GPU
     // row-split matmuls driven from ONE host thread (ggml_backend_split_buffer_type): a context + join event per peer device
     b200_ctx *    split_peer[16] = {nullptr};
@@ -179,7 +166,7 @@ int op_allreduce(b200_ctx *ctx, const b200_op *op);     // comm.cu
 bool supports_allreduce(const b200_op *op);
 int comm_check(b200_ctx *ctx);                          // comm.cu: B200_ERR_FAILED if an all-reduce timed out waiting for a peer
 
-// rope parameters shared by glue.cu and the decode-step kernel (dstep.cu)
+// rope parameters of the rope and rope+store kernels (glue.cu)
 struct RopeParams {
     int n_dims, mode, n_ctx_orig;
     float freq_base, freq_scale, ext_factor, attn_factor, beta_fast, beta_slow;
@@ -187,7 +174,6 @@ struct RopeParams {
     int exact;        // cpu-exact mode: glibc's sinf/cosf restated (common.cuh), which the CPU backend calls; CUDA's sinf/cosf are
                       // 1-2 ulp off here and there and every ulp can flip a KV-store / activation rounding downstream
 };
-RopeParams make_rope_params(const int32_t *params);      // glue.cu: op_params words -> RopeParams (theta_scale, YaRN corr dims)
 
 // fused ROPE(q) + ROPE(k) + KV-store of k and v for a decode ubatch (glue.cu); q/k/v are contiguous [D, heads, T] f32
 struct RopeStoreDesc {

@@ -35,8 +35,6 @@ struct FaParams {
     const char *mask; uint64_t m_nb1;
     float *dst;
     float *part;                 // [tile][split][16][D + 2]
-    int *counters;               // [tile] arrivals of the KV splits (self-resetting); NULL: separate combine kernel
-    int cluster;                 // 1: the KV splits of a tile form a thread-block cluster and are merged through distributed shared memory (no partial buffer, no combine kernel)
     const int *map; int map_stride;   // live-tile map [n_coltiles][1 + n_kv / 32]: count, then the indices of the 32-position tiles with any unmasked cell
     int n_q, n_kv, H, Hkv, gq, HG, QC, n_headtiles, n_coltiles, n_splits, kv_per_split;
     float scale, softcap, max_bias, m0, m1;
@@ -58,9 +56,6 @@ __device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], 
 __device__ __forceinline__ void cp_async16(void *s, const void *g) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(s)), "l"(g));
 }
-__device__ __forceinline__ uint32_t fa_mapa(uint32_t addr, uint32_t rank) { uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank)); return r; }
-__device__ __forceinline__ float fa_ld_cluster(uint32_t addr) { float v; asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(addr)); return v; }
-__device__ __forceinline__ void fa_cluster_sync() { asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
     const __half2 h = __floats2half2_rn(a, b);
@@ -140,8 +135,8 @@ __device__ __forceinline__ void fetch_raw(uint8_t *rawbuf, const char *g, uint64
     }
 }
 
-// merge the per-warp results of a CTA (cm / cl / co in shared memory, rows r of the tile; fixed warp order), then write the result, the
-// split partial, or merge the splits (cluster / last-arriver variants).  Shared by the 16-row kernel and the few-row kernel.
+// merge the per-warp results of a CTA (cm / cl / co in shared memory, rows r of the tile; fixed warp order), then write the result or,
+// with several KV splits, the split partial for the combine kernel.  Shared by the 16-row kernel and the few-row kernel.
 template <int D>
 __device__ __forceinline__ void fa_merge_store(const FaParams &p, uint8_t *fsm, int ht, int hk, int c0, int split) {
     float *cm = (float *)fsm;             // [NWARP][16] max
@@ -172,79 +167,10 @@ __device__ __forceinline__ void fa_merge_store(const FaParams &p, uint8_t *fsm, 
         const bool valid = (r / p.HG) < p.QC && col < p.n_q && hin < p.gq;
         if (p.n_splits == 1) {
             if (valid) p.dst[((uint64_t)col * p.H + hk * p.gq + hin) * D + d] = val / L;
-        } else if (p.cluster) {
-            float *cx = co + NWARP * 16 * D;                   // this split's merged tile [16][D + 2], read by cluster rank 0
-            cx[r * (D + 2) + d] = val;
-            if (d == 0) { cx[r * (D + 2) + D] = M; cx[r * (D + 2) + D + 1] = L; }
         } else {
             float *pp = p.part + (((uint64_t)tile_id * p.n_splits + split) * 16 + r) * (D + 2);
             pp[d] = val;
             if (d == 0) { pp[D] = M; pp[D + 1] = L; }
-        }
-    }
-    // ---- cluster mode: the splits of this tile are the CTAs of one cluster; rank 0 merges them (log-sum-exp, fixed split order) straight
-    //      out of the other CTAs' shared memory.  One launch instead of two and no partial round trip through global memory.
-    if (p.n_splits > 1 && p.cluster) {
-        float *cx = co + NWARP * 16 * D;
-        float *fac = cx + 16 * (D + 2);                        // [16][8] per-split weights exp(M_sp - M) / Lsum of every row
-        fa_cluster_sync();
-        if (split == 0) {
-            const uint32_t cx_s = smem_u32(cx);
-            if (threadIdx.x < 16) {
-                const int r = threadIdx.x;
-                float Ms[8], Mx = -INFINITY, Lsum = 0.0f;
-                for (int sp = 0; sp < p.n_splits; sp++) { Ms[sp] = fa_ld_cluster(fa_mapa(cx_s + (uint32_t)(r * (D + 2) + D) * 4, sp)); Mx = fmaxf(Mx, Ms[sp]); }
-                for (int sp = 0; sp < p.n_splits; sp++) {
-                    const float f = Ms[sp] == -INFINITY ? 0.0f : expf(Ms[sp] - Mx);
-                    Lsum += fa_ld_cluster(fa_mapa(cx_s + (uint32_t)(r * (D + 2) + D + 1) * 4, sp)) * f;
-                    fac[r * 8 + sp] = f;
-                }
-                fac[16 * 8 + r] = Lsum;
-            }
-            __syncthreads();
-            for (int e = threadIdx.x; e < 16 * D; e += NWARP * 32) {
-                const int r = e / D, d = e % D;
-                const int hin = ht * p.HG + r % p.HG, col = c0 + r / p.HG;
-                if (!((r / p.HG) < p.QC && col < p.n_q && hin < p.gq)) continue;
-                float acc = 0.0f;
-                for (int sp = 0; sp < p.n_splits; sp++) acc += fa_ld_cluster(fa_mapa(cx_s + (uint32_t)(r * (D + 2) + d) * 4, sp)) * fac[r * 8 + sp];
-                p.dst[((uint64_t)col * p.H + hk * p.gq + hin) * D + d] = acc / fac[16 * 8 + r];
-            }
-        }
-        fa_cluster_sync();                                     // nobody leaves while rank 0 still reads its shared memory
-        return;
-    }
-    // ---- the LAST split of a tile to arrive merges all splits (log-sum-exp, fixed split order => deterministic):
-    //      saves the combine kernel and its launch boundary on the decode critical path ----
-    if (p.n_splits > 1 && p.counters) {
-        __shared__ int s_last;
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            const int prev = atomicAdd(&p.counters[tile_id], 1);
-            s_last = prev == p.n_splits - 1;
-            if (s_last) p.counters[tile_id] = 0;           // ready for the next launch (CUDA-graph replay)
-        }
-        __syncthreads();
-        if (!s_last) return;
-        __threadfence();
-        const float *base = p.part + (uint64_t)tile_id * p.n_splits * 16 * (D + 2);
-        const uint64_t sstride = (uint64_t)16 * (D + 2);
-        for (int e = threadIdx.x; e < 16 * D; e += NWARP * 32) {
-            const int r = e / D, d = e % D;
-            const int hin = ht * p.HG + r % p.HG, col = c0 + r / p.HG;
-            if (!((r / p.HG) < p.QC && col < p.n_q && hin < p.gq)) continue;
-            const float *rp = base + (uint64_t)r * (D + 2);
-            float M = -INFINITY;
-            for (int sp = 0; sp < p.n_splits; sp++) M = fmaxf(M, __ldcg(rp + sp * sstride + D));
-            float Lsum = 0.0f, acc = 0.0f;
-            for (int sp = 0; sp < p.n_splits; sp++) {
-                const float ms = __ldcg(rp + sp * sstride + D);
-                const float f = ms == -INFINITY ? 0.0f : expf(ms - M);
-                Lsum += __ldcg(rp + sp * sstride + D + 1) * f;
-                acc += __ldcg(rp + sp * sstride + d) * f;
-            }
-            p.dst[((uint64_t)col * p.H + hk * p.gq + hin) * D + d] = acc / Lsum;
         }
     }
 }
@@ -806,126 +732,6 @@ __global__ void __launch_bounds__(128) b200_fattn_maskmap_kernel(const char *mas
     }
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// Single-token decode over an f16 cache: a vector kernel (replaces flash_attn_vec_ext_f32, fattn-vec-f32.cuh:4-282, for the
-// bs1 step, where the 16-row mma tile above is a quarter full and its fixed costs dominate 3 MB of KV).  One WARP = one
-// 32-position tile of one KV head = one KV split; all `gq` query heads of the group share every K/V byte.
-//   S = Q.K : lane j owns position j; Q is rounded to f16 like the CPU does for an f16 K (products exact, f32 accumulate)
-//   softmax : one tile per warp -> plain max / sum over the 32 lanes, no running rescale
-//   O = P.V : lane owns 4 of the 128 dims; p_j of every head is broadcast by shuffle, V rows are read coalesced, f32 accumulate
-// K and V tiles are prefetched into L2 BEFORE griddepcontrol.wait (L2 is coherent with the rope+store kernel's writes).
-// Partials go to the same [tile][split][16][D+2] layout, merged by b200_fattn_combine_kernel.
-template <int GQ>
-__global__ void __launch_bounds__(NWARP * 32) b200_fattn_vec_kernel(const FaParams p) {
-    constexpr int D = 128;
-    constexpr int KLD = D * 2 + 16;                        // bytes per staged K row: +16 keeps lane-strided 128-bit reads conflict-free
-    extern __shared__ __align__(128) uint8_t vsm[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint8_t *wsm = vsm + (size_t)warp * (BK * KLD + BK * D * 2 + GQ * D * 4);
-    uint8_t *sK = wsm, *sV = wsm + BK * KLD;
-    float *sq = (float *)(sV + BK * D * 2);               // f16-rounded Q of the group [GQ][D], per warp (no CTA-wide sync anywhere)
-    const int split = blockIdx.x * NWARP + warp, hk = blockIdx.y;
-    const int p0 = split * BK;
-    const bool active = split < p.n_splits;
-    const char *kbase = p.k + (uint64_t)hk * p.k_nb2 + (uint64_t)p0 * p.k_nb1;
-    const char *vbase = p.v + (uint64_t)hk * p.v_nb2 + (uint64_t)p0 * p.v_nb1;
-    if (active) {      // warm the L2 while the producer kernels are still running
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(kbase + (uint64_t)lane * p.k_nb1));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(kbase + (uint64_t)lane * p.k_nb1 + 128));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(vbase + (uint64_t)lane * p.v_nb1));
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(vbase + (uint64_t)lane * p.v_nb1 + 128));
-    }
-    if (p.use_pdl) { pdl_trigger(); pdl_wait(); }
-    if (!active) return;
-    float *pp = p.part + (((uint64_t)hk * p.n_splits + split) * 16) * (D + 2);
-    // mask of my position (query column 0); a fully masked tile contributes nothing
-    const __half mh = *(const __half *)(p.mask + (uint64_t)(p0 + lane) * 2);
-    const float mval = __half2float(mh);
-    const bool masked = __hisinf(mh) && mval < 0.0f;
-    if (__all_sync(0xffffffffu, masked)) {
-        if (lane < p.gq) { pp[(uint64_t)lane * (D + 2) + D] = -INFINITY; pp[(uint64_t)lane * (D + 2) + D + 1] = 0.0f; }
-        return;
-    }
-    // ---- stage the K and V tiles with coalesced 16-byte async copies: every byte of the tile is in flight at once ----
-    {
-        const int half = lane >> 4, c16 = lane & 15;      // two rows per instruction, 16 chunks of 16 bytes per row
-#pragma unroll
-        for (int r = 0; r < BK; r += 2) {
-            const int row = r + half;
-            cp_async16(sK + row * KLD + c16 * 16, kbase + (uint64_t)row * p.k_nb1 + c16 * 16);
-            cp_async16(sV + row * (D * 2) + c16 * 16, vbase + (uint64_t)row * p.v_nb1 + c16 * 16);
-        }
-    }
-    // Q -> f16-rounded f32 in shared memory (overlaps the copies)
-#pragma unroll
-    for (int h = 0; h < GQ; h++) {
-        if (h < p.gq) {
-            const float4 q4 = *(const float4 *)(p.q + (uint64_t)(hk * p.gq + h) * p.q_nb2 + (uint64_t)lane * 16);
-            float4 r;
-            r.x = __half2float(__float2half_rn(q4.x)); r.y = __half2float(__float2half_rn(q4.y));
-            r.z = __half2float(__float2half_rn(q4.z)); r.w = __half2float(__float2half_rn(q4.w));
-            *(float4 *)&sq[h * D + lane * 4] = r;
-        }
-    }
-    cp_async_wait_all();
-    __syncwarp();
-    // ---- S = Q.K for my position (lane j owns position j) ------------------------------------------------------
-    float sc[GQ];
-#pragma unroll
-    for (int h = 0; h < GQ; h++) sc[h] = 0.0f;
-    const uint8_t *krow = sK + lane * KLD;
-#pragma unroll 4
-    for (int c = 0; c < D / 8; c++) {
-        const uint4 kq = *(const uint4 *)(krow + c * 16);
-        const float2 k0 = __half22float2(*(const __half2 *)&kq.x), k1 = __half22float2(*(const __half2 *)&kq.y);
-        const float2 k2 = __half22float2(*(const __half2 *)&kq.z), k3 = __half22float2(*(const __half2 *)&kq.w);
-#pragma unroll
-        for (int h = 0; h < GQ; h++) {
-            if (h < p.gq) {
-                const float4 qa = *(const float4 *)&sq[h * D + c * 8], qb = *(const float4 *)&sq[h * D + c * 8 + 4];
-                float a = sc[h];
-                a = fmaf(qa.x, k0.x, a); a = fmaf(qa.y, k0.y, a); a = fmaf(qa.z, k1.x, a); a = fmaf(qa.w, k1.y, a);
-                a = fmaf(qb.x, k2.x, a); a = fmaf(qb.y, k2.y, a); a = fmaf(qb.z, k3.x, a); a = fmaf(qb.w, k3.y, a);
-                sc[h] = a;
-            }
-        }
-    }
-    // ---- softmax over the tile ---------------------------------------------------------------------------------
-    float pj[GQ], Mh[GQ], Lh[GQ];
-#pragma unroll
-    for (int h = 0; h < GQ; h++) {
-        const float sv = masked ? -INFINITY : sc[h] * p.scale + mval;
-        const float M = warp_reduce_max(sv);
-        const float e = (masked || M == -INFINITY) ? 0.0f : expf(sv - M);
-        pj[h] = e; Mh[h] = M; Lh[h] = warp_reduce_sum(e);
-    }
-    // ---- O = P.V : lane owns dims [4*lane, 4*lane+4) -------------------------------------------------------------
-    float o[GQ][4];
-#pragma unroll
-    for (int h = 0; h < GQ; h++) o[h][0] = o[h][1] = o[h][2] = o[h][3] = 0.0f;
-#pragma unroll 8
-    for (int j = 0; j < BK; j++) {
-        const uint2 vv = *(const uint2 *)(sV + j * (D * 2) + lane * 8);
-        const float2 v0 = __half22float2(*(const __half2 *)&vv.x), v1 = __half22float2(*(const __half2 *)&vv.y);
-#pragma unroll
-        for (int h = 0; h < GQ; h++) {
-            if (h < p.gq) {
-                const float w = __shfl_sync(0xffffffffu, pj[h], j);
-                o[h][0] = fmaf(w, v0.x, o[h][0]); o[h][1] = fmaf(w, v0.y, o[h][1]); o[h][2] = fmaf(w, v1.x, o[h][2]); o[h][3] = fmaf(w, v1.y, o[h][3]);
-            }
-        }
-    }
-#pragma unroll
-    for (int h = 0; h < GQ; h++) {
-        if (h < p.gq) {
-            float *row = pp + (uint64_t)h * (D + 2);
-            *(float2 *)(row + lane * 4) = make_float2(o[h][0], o[h][1]);          // rows are (D + 2) floats apart: 8-byte aligned only
-            *(float2 *)(row + lane * 4 + 2) = make_float2(o[h][2], o[h][3]);
-            if (lane == 0) { row[D] = Mh[h]; row[D + 1] = Lh[h]; }
-        }
-    }
-}
-
 // merge of the KV splits: one WARP per (tile, query row); lanes first reduce the per-split (max, sum) pairs, then each lane
 // owns D/32 output dims and walks the splits with independent loads (log-sum-exp merge, fixed split order => deterministic)
 template <int D>
@@ -1163,7 +969,7 @@ int launch_fa(b200_ctx *ctx, const FaParams &p, int n_tiles) {
     constexpr int LD = D + 8;
     constexpr int RAWK = KT != KV_F16 ? BK * (KT == KV_Q8_0 ? 34 : 18) * (D / 32) : 0, RAWV = VT != KV_F16 ? BK * (VT == KV_Q8_0 ? 34 : 18) * (D / 32) : 0;
     constexpr int WARP_BYTES = 2 * BK * LD * 2 + 2 * BK * (D / 32) * 4 + RAWK + RAWV + (ROWS8 ? 2 * 8 * 40 * 2 : 0);
-    constexpr int COMBINE_BYTES = (2 * NWARP * 16 + NWARP * 16 * D + 16 * (D + 2) + 16 * 8 + 16) * 4;      // warp merge + cluster merge areas
+    constexpr int COMBINE_BYTES = (2 * NWARP * 16 + NWARP * 16 * D) * 4;      // warp merge area (fa_merge_store)
     constexpr int SMEM = NWARP * WARP_BYTES > COMBINE_BYTES ? NWARP * WARP_BYTES : COMBINE_BYTES;
     auto kern = ROWS8 ? b200_fattn_rows8_kernel<D, KT, VT> : b200_fattn_kernel<D, KT, VT>;
     static bool attr_set[16] = {false};
@@ -1171,10 +977,9 @@ int launch_fa(b200_ctx *ctx, const FaParams &p, int n_tiles) {
         CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
         attr_set[ctx->device & 15] = true;
     }
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     int na = 0;
     if (p.use_pdl) { attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[na].val.programmaticStreamSerializationAllowed = 1; na++; }
-    if (p.cluster) { attr[na].id = cudaLaunchAttributeClusterDimension; attr[na].val.clusterDim.x = (unsigned)p.n_splits; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1; na++; }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)p.n_splits, (unsigned)n_tiles);
     cfg.blockDim = dim3(NWARP * 32);
@@ -1184,15 +989,7 @@ int launch_fa(b200_ctx *ctx, const FaParams &p, int n_tiles) {
     cfg.numAttrs = na;
     CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, p));
     ctx->launches++;
-    if (p.cluster) return B200_OK;
-    cfg.numAttrs = p.use_pdl ? 1 : 0;
-    if (p.n_splits > 1 && !p.counters) {
-        if (ROWS8 && D == 128 && ctx->fa_skip_combine && p.n_q == 1 && p.n_splits <= 16) {
-            // batch-1 decode: the output projection's GEMV merges the splits in its activation prologue (gemv_bs1.cu bs1_load_fa_partials,
-            // same arithmetic in the same order as b200_fattn_combine_kernel): one launch less on the token's critical path
-            ctx->fa_part = p.part; ctx->fa_part_ns = p.n_splits; ctx->fa_part_gq = p.gq;
-            return B200_OK;
-        }
+    if (p.n_splits > 1) {
         cfg.gridDim = dim3((unsigned)((n_tiles * 16 + 3) / 4));
         cfg.blockDim = dim3(128);
         cfg.dynamicSmemBytes = 0;
@@ -1303,43 +1100,6 @@ int op_flash_attn_ext(b200_ctx *ctx, const b200_op *op) {
         a.mask = p.mask; a.m_nb1 = p.m_nb1; a.dst = p.dst; a.n_q = p.n_q; a.n_kv = p.n_kv; a.H = p.H; a.gq = p.gq; a.scale = p.scale;
         return fattn_tc_launch(ctx, a, kv_kind(k.type));
     }
-    // single-token decode over an f16 cache: the vector kernel (one warp per 32 positions, all heads of the group).  Parity green,
-    // but measured SLOWER than the mma tile kernel in round 1 (10.5 + 9.2 us with 24 splits to merge vs 9.5 + 5.1 us; 499 vs
-    // 536 tok/s on Llama-3-8B bs1), so it is opt-in until its latency chain is understood (DESIGN.md 7)
-    static const int use_vec = getenv("GGML_B200_FA_VEC") ? atoi(getenv("GGML_B200_FA_VEC")) : 0;
-    if (use_vec && p.n_q == 1 && D == 128 && kv_kind(k.type) == KV_F16 && kv_kind(v.type) == KV_F16 && p.gq <= 8 && has_mask &&
-        p.softcap == 0.0f && p.max_bias == 0.0f && !(q.nb[2] & 15) && !((uintptr_t)q.data & 15) && !(v.nb[1] & 7) && !(k.nb[1] & 15)) {
-        p.n_splits = p.n_kv / BK;
-        p.kv_per_split = BK;
-        p.part = (float *)ctx->get_scratch(SCRATCH_FATTN, (size_t)n_tiles * p.n_splits * 16 * (D + 2) * 4);
-        if (!p.part) return B200_ERR_ALLOC;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)((p.n_splits + NWARP - 1) / NWARP), (unsigned)p.Hkv);
-        cfg.blockDim = dim3(NWARP * 32);
-        cfg.stream = ctx->stream;
-        cfg.attrs = attr;
-        cfg.numAttrs = p.use_pdl ? 1 : 0;
-        const int GQv = p.gq <= 4 ? 4 : 8;
-        cfg.dynamicSmemBytes = (size_t)NWARP * (BK * (128 * 2 + 16) + BK * 128 * 2 + GQv * 128 * 4);
-        static bool vattr[16] = {false};
-        if (!vattr[ctx->device & 15]) {
-            CUDA_TRY(cudaFuncSetAttribute(b200_fattn_vec_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-            CUDA_TRY(cudaFuncSetAttribute(b200_fattn_vec_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-            vattr[ctx->device & 15] = true;
-        }
-        if (p.gq <= 4) CUDA_TRY(cudaLaunchKernelEx(&cfg, b200_fattn_vec_kernel<4>, p));
-        else CUDA_TRY(cudaLaunchKernelEx(&cfg, b200_fattn_vec_kernel<8>, p));
-        cfg.dynamicSmemBytes = 0;
-        ctx->launches++;
-        cfg.gridDim = dim3((unsigned)((n_tiles * 16 + 3) / 4));
-        cfg.blockDim = dim3(128);
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, b200_fattn_combine_kernel<128>, p, n_tiles));
-        ctx->launches++;
-        return B200_OK;
-    }
     // batched steps and prompt ubatches: live-tile map of the mask, shared by every layer of the graph
     static const int use_map = getenv("GGML_B200_FA_MAP") ? atoi(getenv("GGML_B200_FA_MAP")) : 1;
     if (use_map && has_mask && p.n_q > 1 && p.n_kv / BK <= 4 * MAP_MAX_BATCH * 32 && !((uintptr_t)m.data & 15) && !(m.nb[1] & 15)) {
@@ -1375,24 +1135,11 @@ int op_flash_attn_ext(b200_ctx *ctx, const b200_op *op) {
     p.kv_per_split = ((p.n_kv + ns - 1) / ns + unit - 1) / unit * unit;
     ns = (p.n_kv + p.kv_per_split - 1) / p.kv_per_split;
     p.n_splits = ns;
-    // 2..8 splits CAN form one thread-block cluster per tile and merge through distributed shared memory (one launch, no partials; opt-in)
-    static const int use_cluster = getenv("GGML_B200_FA_CLUSTER") ? atoi(getenv("GGML_B200_FA_CLUSTER")) : 0;   // measured slower than the PDL combine kernel (511 vs 529 tok/s bs1): opt-in
-    p.cluster = use_cluster && ns >= 2 && ns <= 8;
-    if (ns > 1 && !p.cluster) {
+    if (ns > 1) {
         // sized by its upper bound (n_tiles * ns <= 4 * sm_count + n_tiles) so that a growing n_kv never reallocates it under
         // captured graphs
         p.part = (float *)ctx->get_scratch(SCRATCH_FATTN, (size_t)(4 * ctx->sm_count + n_tiles) * 16 * (D + 2) * 4);
         if (!p.part) return B200_ERR_ALLOC;
-        // merging the splits in the last-arriving CTA instead of a second kernel was measured SLOWER on B200 (471 vs 523 tok/s on
-        // Llama-3-8B bs1: a PDL kernel boundary costs ~1 us, the serialised fence + atomic + 128-thread merge costs more): off
-        static const int fuse_combine = getenv("GGML_B200_FA_FUSED_COMBINE") ? atoi(getenv("GGML_B200_FA_FUSED_COMBINE")) : 0;
-        if (fuse_combine && n_tiles <= 4096) {
-            if (!ctx->fattn_counters) {       // zeroed once; the kernel leaves every counter at zero again
-                if (cudaMalloc(&ctx->fattn_counters, 4096 * sizeof(int)) != cudaSuccess) { cudaGetLastError(); ctx->fattn_counters = nullptr; }
-                else CUDA_TRY(cudaMemset(ctx->fattn_counters, 0, 4096 * sizeof(int)));
-            }
-            p.counters = (int *)ctx->fattn_counters;
-        }
     }
     const int kt = kv_kind(k.type), vt = kv_kind(v.type);
     if (D == 128) return launch_fa_types<128>(ctx, p, n_tiles, kt, vt, rows8);

@@ -1,7 +1,7 @@
 // gemm_mma.cu -- prompt-batch GEMM (more than 32 token columns) for all five GGUF formats on the warp-level tensor-core path.
 //
 // Replaces mul_mat_q (ggml-cuda/mmq.cuh:2501-2657: 128 x mmq_x tiles, weights de-nibbled to int8 in shared memory, q8_1 activations,
-// float fix-up per 32-k block).  Round-1's tcgen05 GEMM (gemm_i8.cu) keeps the tensor pipe 6 % busy: its CUDA-core stages -- expanding
+// float fix-up per 32-k block).  Round 1's tcgen05 kind::i8 GEMM (since removed) kept the tensor pipe 6 % busy: its CUDA-core stages -- expanding
 // every weight block to hi/lo int8 operand tiles once per 128-token tile, and a ~16-instruction drain per output element per
 // 256 k -- bound it at 112 TOPS, below the reference's own MMQ on the same B200 (profiles/r2_ref_cuda_vs_plugin.txt).  This kernel
 // removes both stages:
@@ -27,13 +27,13 @@ constexpr int G_THREADS = 8 * 32;                     // 8 warps: 255 registers 
 
 // stage image of the activations of one (token tile, super-block), written by the pack kernel, copied by one bulk copy:
 //   [128 tokens][272] int8 quants | d: q8_K [128] floats, q8_0 mode [128][8] floats | q8_K only: per-32 sums [128][8] int16
-// (tn = tokens per tile: 128, or 64 for the two-CTAs-per-SM variant)
-__host__ __device__ inline uint32_t img_off_d(int tn) { return tn * G_BSTRIDE; }
-__host__ __device__ inline uint32_t img_off_s(int q8k, int tn) { return img_off_d(tn) + (q8k ? tn * 4 : tn * 8 * 4); }
-__host__ __device__ inline uint32_t img_bytes(int q8k, int tn) { return (img_off_s(q8k, tn) + (q8k ? tn * 8 * 2 : 0) + 127u) & ~127u; }
+__host__ __device__ inline uint32_t img_off_d() { return GT_N * G_BSTRIDE; }
+__host__ __device__ inline uint32_t img_off_s(int q8k) { return img_off_d() + (q8k ? GT_N * 4 : GT_N * 8 * 4); }
+__host__ __device__ inline uint32_t img_bytes(int q8k) { return (img_off_s(q8k) + (q8k ? GT_N * 8 * 2 : 0) + 127u) & ~127u; }
 
 struct GParams {
-    const uint8_t *W; uint32_t rb, bbytes; int type, N, K, M, q8k, tn;
+    const uint8_t *W; uint32_t rb, bbytes; int type, N, K, M, q8k;
+    int tn;                                            // = GT_N.  g_lookup reads it from here: with the constant folded in, ptxas spills twice as much in the Q5_K GEMM
     const uint8_t *img;                                // [ntile][nsb] stage images
     float *dst; size_t dst_stride;
     float *part;                                       // [ksplit][M][N] when ksplit > 1
@@ -70,13 +70,13 @@ __device__ __forceinline__ float hf(uint32_t bits) { return __half2float(__ushor
 
 // ---------------------------------------------------------------------------------------------------------------- activation pack
 // one warp per (token, super-block): quantise 256 floats like the CPU and write them into the stage image of the token's tile
-__global__ void __launch_bounds__(256) b200_gemm_mma_pack_kernel(const float *__restrict__ x, size_t x_stride, int K, int M, int q8k, int nsb, int tn, uint8_t *__restrict__ img) {
+__global__ void __launch_bounds__(256) b200_gemm_mma_pack_kernel(const float *__restrict__ x, size_t x_stride, int K, int M, int q8k, int nsb, uint8_t *__restrict__ img) {
     const int lane = threadIdx.x & 31;
     const int64_t gw = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
-    const int ntile = (M + tn - 1) / tn;
-    if (gw >= (int64_t)ntile * tn * nsb) return;
-    const int b = (int)(gw % nsb), tok = (int)(gw / nsb), tile = tok / tn, t = tok % tn;
-    uint8_t *im = img + ((size_t)tile * nsb + b) * img_bytes(q8k, tn);
+    const int ntile = (M + GT_N - 1) / GT_N;
+    if (gw >= (int64_t)ntile * GT_N * nsb) return;
+    const int b = (int)(gw % nsb), tok = (int)(gw / nsb), tile = tok / GT_N, t = tok % GT_N;
+    uint8_t *im = img + ((size_t)tile * nsb + b) * img_bytes(q8k);
     float v[8];
     if (tok < M) {
         const float *xp = (const float *)((const char *)x + (size_t)tok * x_stride) + b * 256 + lane * 8;
@@ -91,12 +91,12 @@ __global__ void __launch_bounds__(256) b200_gemm_mma_pack_kernel(const float *__
         float d; int pair;
         warp_quant_q8k(v, lane, qp, d, pair);
         const int s32 = pair + __shfl_down_sync(0xffffffffu, pair, 2);           // even lanes hold per-16 sums: lanes 0, 4, 8, ... add their neighbour pair
-        if ((lane & 3) == 0) ((int16_t *)(im + img_off_s(1, tn)))[t * 8 + (lane >> 2)] = (int16_t)s32;
-        if (lane == 0) ((float *)(im + img_off_d(tn)))[t] = d;
+        if ((lane & 3) == 0) ((int16_t *)(im + img_off_s(1)))[t * 8 + (lane >> 2)] = (int16_t)s32;
+        if (lane == 0) ((float *)(im + img_off_d()))[t] = d;
     } else {
         float d16; int bsum;
         warp_quant_q80(v, qp, d16, bsum);
-        if ((lane & 3) == 0) ((float *)(im + img_off_d(tn)))[t * 8 + (lane >> 2)] = d16;
+        if ((lane & 3) == 0) ((float *)(im + img_off_d()))[t * 8 + (lane >> 2)] = d16;
     }
     *(uint2 *)(im + (size_t)t * G_BSTRIDE + lane * 8) = qp;
 }
@@ -285,13 +285,12 @@ __device__ __forceinline__ void sb_compute(const uint8_t *const (&rowp)[2][2], u
 __global__ void __launch_bounds__(256) b200_gemm_mma_pack_grouped_kernel(const float *__restrict__ x, size_t x_stride, GParams p, uint8_t *__restrict__ img) {
     const int lane = threadIdx.x & 31;
     const int64_t gw = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
-    const int tn = p.tn;
-    if (gw >= (int64_t)p.g_chunks * tn * p.nsb) return;
-    const int b = (int)(gw % p.nsb), slot = (int)(gw / p.nsb), chunk = slot / tn, t = slot % tn;
+    if (gw >= (int64_t)p.g_chunks * GT_N * p.nsb) return;
+    const int b = (int)(gw % p.nsb), slot = (int)(gw / p.nsb), chunk = slot / GT_N, t = slot % GT_N;
     int e, first, cnt;
     g_lookup(p, chunk, e, first, cnt);
     if (cnt == 0) return;
-    uint8_t *im = img + ((size_t)chunk * p.nsb + b) * img_bytes(p.q8k, tn);
+    uint8_t *im = img + ((size_t)chunk * p.nsb + b) * img_bytes(p.q8k);
     float v[8];
     if (t < cnt) {
         const int pair = p.g_pairs[first + t];
@@ -308,20 +307,20 @@ __global__ void __launch_bounds__(256) b200_gemm_mma_pack_grouped_kernel(const f
         float d; int pair;
         warp_quant_q8k(v, lane, qp, d, pair);
         const int s32 = pair + __shfl_down_sync(0xffffffffu, pair, 2);
-        if ((lane & 3) == 0) ((int16_t *)(im + img_off_s(1, tn)))[t * 8 + (lane >> 2)] = (int16_t)s32;
-        if (lane == 0) ((float *)(im + img_off_d(tn)))[t] = d;
+        if ((lane & 3) == 0) ((int16_t *)(im + img_off_s(1)))[t * 8 + (lane >> 2)] = (int16_t)s32;
+        if (lane == 0) ((float *)(im + img_off_d()))[t] = d;
     } else {
         float d16; int bsum;
         warp_quant_q80(v, qp, d16, bsum);
-        if ((lane & 3) == 0) ((float *)(im + img_off_d(tn)))[t * 8 + (lane >> 2)] = d16;
+        if ((lane & 3) == 0) ((float *)(im + img_off_d()))[t * 8 + (lane >> 2)] = d16;
     }
     *(uint2 *)(im + (size_t)t * G_BSTRIDE + lane * 8) = qp;
 }
 
 // ---------------------------------------------------------------------------------------------------------------- the GEMM
-template <int TYPE, int TN>
-__global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_kernel(const GParams p) {
-    constexpr int NTW = TN / 16;                      // n-tiles per warp: the two token halves of the tile belong to warps wn = 0, 1
+template <int TYPE>
+__global__ void __launch_bounds__(G_THREADS, 1) b200_gemm_mma_kernel(const GParams p) {
+    constexpr int NTW = GT_N / 16;                      // n-tiles per warp: the two token halves of the tile belong to warps wn = 0, 1
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t *full = (uint64_t *)smem, *empty = full + 8;
     uint8_t *ring = smem + 128;
@@ -332,7 +331,7 @@ __global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_ker
         mbar_fence_init();
     }
     __syncthreads();
-    const uint32_t ibytes = img_bytes(p.q8k, TN);
+    const uint32_t ibytes = img_bytes(p.q8k);
 
     // ------------------------------------------------------------ producer side, ALL threads: stage iteration p_it stands for (p_item, p_b).
     // The 128 row pieces of a stage (144..272 bytes each) go through 16-byte cp.async issued by every thread -- a bulk copy per piece
@@ -381,7 +380,7 @@ __global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_ker
         const int ks = item % p.ksplit, rt = (item / p.ksplit) % p.nrt, tt = item / (p.ksplit * p.nrt);
         const int sb0 = ks * p.sb_per_split, sb1 = min(p.nsb, sb0 + p.sb_per_split);
         const uint8_t *Wc = p.W;
-        int g_first = 0, g_cnt = TN;
+        int g_first = 0, g_cnt = GT_N;
         if (p.g_E) {
             int e;
             g_lookup(p, tt, e, g_first, g_cnt);
@@ -399,9 +398,9 @@ __global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_ker
             mbar_wait(&full[st], (it / ns) & 1);
             const uint8_t *stage = ring + (size_t)st * p.stage_bytes;
             const uint8_t *bimg = stage + p.a_bytes;
-            const uint32_t bq = smem_u32(bimg) + (uint32_t)(wn * (TN / 2)) * G_BSTRIDE;
-            const float *bd = (const float *)(bimg + img_off_d(TN));
-            const int16_t *bs = (const int16_t *)(bimg + img_off_s(p.q8k, TN));
+            const uint32_t bq = smem_u32(bimg) + (uint32_t)(wn * (GT_N / 2)) * G_BSTRIDE;
+            const float *bd = (const float *)(bimg + img_off_d());
+            const int16_t *bs = (const int16_t *)(bimg + img_off_s(p.q8k));
             // B fragment address of this lane for ldmatrix.x4 over two n-tiles: matrix mi = lane >> 3 -> (n-tile pair member, k half)
             const uint32_t b_lane = bq + (uint32_t)(((lane >> 4) & 1) * 8 + (lane & 7)) * G_BSTRIDE + (uint32_t)((lane >> 3) & 1) * 16;
             const uint8_t *rowp[2][2];
@@ -413,7 +412,7 @@ __global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_ker
                     const uintptr_t g = (uintptr_t)(Wc + (size_t)(rt * GT_M + r) * p.rb + (size_t)b * p.bbytes);
                     rowp[mt][h] = stage + (size_t)r * p.rstride + (g & 15);
                 }
-            sb_compute<TYPE, NTW>(rowp, b_lane, bd, bs, wn * (TN / 2), lane, out);
+            sb_compute<TYPE, NTW>(rowp, b_lane, bd, bs, wn * (GT_N / 2), lane, out);
             __syncwarp();
             if (lane == 0) mbar_arrive(&empty[st]);
         }
@@ -424,7 +423,7 @@ __global__ void __launch_bounds__(G_THREADS, TN == 64 ? 2 : 1) b200_gemm_mma_ker
         for (int nt = 0; nt < NTW; nt++)
 #pragma unroll
             for (int cc = 0; cc < 2; cc++) {
-                const int tl = wn * (TN / 2) + nt * 8 + cq + cc, tok = tt * TN + tl;
+                const int tl = wn * (GT_N / 2) + nt * 8 + cq + cc, tok = tt * GT_N + tl;
                 if (p.g_E) {
                     if (tl < g_cnt) {
                         const int pair = p.g_pairs[g_first + tl];
@@ -450,9 +449,9 @@ __global__ void __launch_bounds__(256) b200_gemm_mma_reduce_kernel(const float *
     dst[(size_t)tok * dst_stride + n] = a;
 }
 
-template <int TYPE, int TN>
-int launch_gt(b200_ctx *ctx, const GParams &p, int grid, size_t smem) {
-    auto kern = b200_gemm_mma_kernel<TYPE, TN>;
+template <int TYPE>
+int launch_g(b200_ctx *ctx, const GParams &p, int grid, size_t smem) {
+    auto kern = b200_gemm_mma_kernel<TYPE>;
     static bool attr_set[16] = {false};
     if (!attr_set[ctx->device & 15]) {
         CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin));
@@ -463,20 +462,13 @@ int launch_gt(b200_ctx *ctx, const GParams &p, int grid, size_t smem) {
     CUDA_TRY(cudaGetLastError());
     return B200_OK;
 }
-template <int TYPE>
-int launch_g(b200_ctx *ctx, const GParams &p, int grid, size_t smem) {
-    return p.tn == 64 ? launch_gt<TYPE, 64>(ctx, p, grid, smem) : launch_gt<TYPE, 128>(ctx, p, grid, smem);
-}
-// tokens per CTA tile: 128 (one CTA per SM, warp tile 32 x 64) or 64 (two CTAs per SM, warp tile 32 x 32)
-static int gemm_tn() { static const int tn = getenv("GGML_B200_GEMM_TN") ? atoi(getenv("GGML_B200_GEMM_TN")) : 128; return tn == 64 ? 64 : 128; }
 // stage geometry + grid shared by the dense and the grouped entry
 static size_t gemm_geometry(b200_ctx *ctx, GParams &p) {
-    const uint32_t ibytes = img_bytes(p.q8k, p.tn);
+    const uint32_t ibytes = img_bytes(p.q8k);
     p.rstride = ((p.bbytes + 15u) & ~15u) + 16;            // >= 16 x chunks per row piece (gemm kernel CPR)
     p.a_bytes = (GT_M * p.rstride + 127u) & ~127u;
     p.stage_bytes = p.a_bytes + ibytes;
-    const size_t budget = p.tn == 64 ? (ctx->smem_optin - 2048) / 2 : ctx->smem_optin;       // tn = 64: two CTAs share the SM
-    int ns = (int)((budget - 128) / p.stage_bytes);
+    int ns = (int)((ctx->smem_optin - 128) / p.stage_bytes);
     if (ns > 4) ns = 4;
     p.nstages = ns;
     return ns < 2 ? 0 : 128 + (size_t)ns * p.stage_bytes;
@@ -495,16 +487,16 @@ int gemm_mma_run(b200_ctx *ctx, int type, const uint8_t *W, size_t rb, int64_t N
     GParams p = {};
     p.W = W; p.rb = (uint32_t)rb; p.type = type; p.N = (int)N; p.K = (int)K; p.M = (int)M; p.q8k = b200_act_mode_q8k(type);
     p.bbytes = type == B200_TYPE_Q4_K ? 144u : type == B200_TYPE_Q5_K ? 176u : type == B200_TYPE_Q6_K ? 210u : type == B200_TYPE_Q4_0 ? 144u : 272u;
-    p.tn = gemm_tn();
-    p.nsb = (int)(K / 256); p.ntile = (int)((M + p.tn - 1) / p.tn); p.nrt = (int)(N / GT_M);
+    p.tn = GT_N;
+    p.nsb = (int)(K / 256); p.ntile = (int)((M + GT_N - 1) / GT_N); p.nrt = (int)(N / GT_M);
     p.dst = dst; p.dst_stride = dst_stride;
-    const uint32_t ibytes = img_bytes(p.q8k, p.tn);
+    const uint32_t ibytes = img_bytes(p.q8k);
     uint8_t *img = (uint8_t *)ctx->get_scratch(SCRATCH_ACT, (size_t)p.ntile * p.nsb * ibytes);
     if (!img) return B200_ERR_ALLOC;
     p.img = img;
     {
-        const int64_t warps = (int64_t)p.ntile * p.tn * p.nsb;
-        b200_gemm_mma_pack_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, ctx->stream>>>(x, x_stride, (int)K, (int)M, p.q8k, p.nsb, p.tn, img);
+        const int64_t warps = (int64_t)p.ntile * GT_N * p.nsb;
+        b200_gemm_mma_pack_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, ctx->stream>>>(x, x_stride, (int)K, (int)M, p.q8k, p.nsb, img);
         ctx->launches++;
         CUDA_TRY(cudaGetLastError());
     }
@@ -513,7 +505,7 @@ int gemm_mma_run(b200_ctx *ctx, int type, const uint8_t *W, size_t rb, int64_t N
     // split K when the tile grid would leave most of the machine idle (slices of >= 4 super-blocks); partials reduced in slice order
     const int64_t tiles = (int64_t)p.nrt * p.ntile;
     int ksplit = 1;
-    while (ksplit < 8 && tiles * ksplit * 2 <= ctx->sm_count * (p.tn == 64 ? 2 : 1) && p.nsb / (ksplit * 2) >= 4) ksplit *= 2;
+    while (ksplit < 8 && tiles * ksplit * 2 <= ctx->sm_count && p.nsb / (ksplit * 2) >= 4) ksplit *= 2;
     p.sb_per_split = (p.nsb + ksplit - 1) / ksplit;
     p.ksplit = (p.nsb + p.sb_per_split - 1) / p.sb_per_split;
     if (p.ksplit > 1) {
@@ -521,8 +513,7 @@ int gemm_mma_run(b200_ctx *ctx, int type, const uint8_t *W, size_t rb, int64_t N
         if (!p.part) return B200_ERR_ALLOC;
     }
     p.nitems = (int)(tiles * p.ksplit);
-    const int slots = ctx->sm_count * (p.tn == 64 ? 2 : 1);
-    const int grid = p.nitems < slots ? p.nitems : slots;
+    const int grid = p.nitems < ctx->sm_count ? p.nitems : ctx->sm_count;
     int rc;
     switch (type) {
         case B200_TYPE_Q4_K: rc = launch_g<B200_TYPE_Q4_K>(ctx, p, grid, smem); break;
@@ -545,17 +536,17 @@ int gemm_mma_run_grouped(b200_ctx *ctx, int type, const uint8_t *W, size_t rb, i
     GParams p = {};
     p.W = W; p.rb = (uint32_t)rb; p.type = type; p.N = (int)N; p.K = (int)K; p.M = 0; p.q8k = b200_act_mode_q8k(type);
     p.bbytes = type == B200_TYPE_Q4_K ? 144u : type == B200_TYPE_Q5_K ? 176u : type == B200_TYPE_Q6_K ? 210u : type == B200_TYPE_Q4_0 ? 144u : 272u;
-    p.tn = 128;
+    p.tn = GT_N;
     p.nsb = (int)(K / 256); p.ntile = g.max_chunks; p.nrt = (int)(N / GT_M);
     p.dst = dst;
     p.g_off = g.off; p.g_pairs = g.pairs; p.g_E = g.E; p.g_n_used = g.n_used; p.g_b_ne1 = g.b_ne1; p.g_chunks = g.max_chunks;
     p.g_expert_stride = g.expert_stride; p.g_d_nb1 = g.d_nb1; p.g_d_nb2 = g.d_nb2;
-    const uint32_t ibytes = img_bytes(p.q8k, p.tn);
+    const uint32_t ibytes = img_bytes(p.q8k);
     uint8_t *img = (uint8_t *)ctx->get_scratch(SCRATCH_ACT, (size_t)p.ntile * p.nsb * ibytes);
     if (!img) return B200_ERR_ALLOC;
     p.img = img;
     {
-        const int64_t warps = (int64_t)p.ntile * p.tn * p.nsb;
+        const int64_t warps = (int64_t)p.ntile * GT_N * p.nsb;
         b200_gemm_mma_pack_grouped_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, ctx->stream>>>(x, x_stride, p, img);
         ctx->launches++;
         CUDA_TRY(cudaGetLastError());

@@ -16,8 +16,8 @@
 //     sums) into a second accumulator.  All values are integers below 2^24 in f32: the CPU's integers, bit for bit;
 //   * the drain warps read both accumulators (tcgen05.ld), and fold  d_a * (d_w * P - dmin_w * Mn)  into f32 registers: three
 //     flops per element per super-block, nothing else -- no hi/lo operand split, no dp2a, no int->float conversion.
-// The round-1 kind::i8 kernel (gemm_i8.cu) needed two operand tiles + two accumulators + a 16-instruction drain per element; the
-// mma.sync kernel (gemm_mma.cu) is bounded by the legacy IMMA pipe and its 4 IMAD per IMMA.  Both stay selectable.
+// The round-1 kind::i8 kernel (measured slower and removed, DESIGN.md 8) needed two operand tiles + two accumulators + a 16-instruction
+// drain per element; the mma.sync kernel (gemm_mma.cu) is bounded by the legacy IMMA pipe and its 4 IMAD per IMMA.
 // Roofline: tensor pipe (f16: half the int8 rate) for prompt batches, HBM for <= 32 tokens.  Algorithmic work: 2*N*K*M.
 #include "common.cuh"
 #include "quant_warp.cuh"

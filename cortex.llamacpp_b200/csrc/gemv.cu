@@ -586,7 +586,6 @@ int gemv_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_t K, con
         if (rc != 0) return rc < 0 ? rc : B200_OK;
         if (pair) *pair = false;
     }
-    if (ga.mode == ACT_FA_PART) { b200_set_error("gemv: flash-attention partials need the batch-1 kernel"); return B200_ERR_UNSUPPORTED; }
     const ActLayout L = ActLayout::make(q8k, K);
     constexpr int MAXW = GEMV_THREADS / 32 - 1;
     const int nwarps = g_gemv_warps > 0 ? (g_gemv_warps > MAXW ? MAXW : g_gemv_warps) : MAXW;

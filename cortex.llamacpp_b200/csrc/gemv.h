@@ -3,7 +3,7 @@
 #include "common.cuh"
 
 constexpr int GEMV_MAX_SEG = 3;
-enum { ACT_PREQ = 0, ACT_F32 = 1, ACT_F32_NORM = 2, ACT_F32_SWIGLU = 3, ACT_FA_PART = 4 };      // ACT_FA_PART: batch-1 kernel only (unmerged flash-attention KV-split partials)
+enum { ACT_PREQ = 0, ACT_F32 = 1, ACT_F32_NORM = 2, ACT_F32_SWIGLU = 3 };
 
 // one weight matrix of a launch ("segment"): dst[:, col] = W . act[:, col] (+ residual)
 struct GemvSegDesc {
@@ -26,8 +26,6 @@ struct GemvActDesc {
     size_t         x_stride;
     const float *  x2;               // ACT_F32_NORM: norm weight [K]; ACT_F32_SWIGLU: `up` (strided like x)
     float          eps;
-    const float *  fa_part = nullptr;   // ACT_FA_PART: partials [kv head][split][16][128 + 2] (fattn.cu), fa_ns splits, fa_gq query heads per KV head
-    int            fa_ns = 0, fa_gq = 0;
 };
 
 // L2 look-ahead: constant weight ranges of the launches that follow this one (graph.cu fills them in)
@@ -40,5 +38,5 @@ int gemv_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_t K, con
 // else; *pair tells the caller whether the launch did it (only the batch-1 kernel can), so that the down projection reads h directly
 // batch-1 K-quant kernel (gemv_bs1.cu): 1 = launched, 0 = not eligible, < 0 = error
 int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_t K, const GemvActDesc &ga, bool w_const,
-                        const GemvPf *pf, int npf, int l2pf, bool *pair = nullptr, bool dry_run = false);
+                        const GemvPf *pf, int npf, int l2pf, bool *pair = nullptr);
 int gemv_max_cols(const b200_ctx *ctx, int type, size_t rb, int64_t K);

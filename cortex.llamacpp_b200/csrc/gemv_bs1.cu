@@ -48,7 +48,6 @@ struct Bs1Params {
     const float *  x, *x2;
     float          eps;
     double         inv_K;                      // 1 / K when K is a power of two (exact), else 0
-    const float *  fa_part; int fa_ns, fa_gq;  // ACT_FA_PART: unmerged flash-attention KV-split partials (see bs1_load_fa_partials)
     int            nstages;
     uint32_t       stage_bytes;
     int            w_const, use_pdl, ncw;      // ncw: consumer warps (blockDim / 32 - 1)
@@ -126,60 +125,6 @@ __device__ __forceinline__ void bs1_apply_mode(const Bs1Params &p, float (&v)[8]
         for (int j = 0; j < 8; j++) v[j] = __fmul_rn(ggml_silu_lane(v[j]), w[j]);
     }
 }
-// ACT_FA_PART: the activation vector is the attention output [head][128] that b200_fattn_combine_kernel would have produced from the
-// KV-split partials part[kv head][split][16 rows][128 + 2] (row = query head inside the GQA group; columns 128 / 129 = running max / sum).
-// Lane owns 8 consecutive dims of one head (a half-warp per head).  Same arithmetic in the same order as the combine kernel -- max over
-// the splits, sum of l_s * expf(m_s - M) by the xor tree (one split per lane, zeros elsewhere), acc += o_s * expf(m_s - M) in split
-// order, acc / L -- so the vector is bit-identical to the unfused path.  Needs fa_ns <= 16.
-__device__ __forceinline__ void bs1_load_fa_partials(const Bs1Params &p, int b, int lane, float4 &v0, float4 &v1) {
-    const int e0 = b * 256 + lane * 8, head = e0 >> 7, d0 = e0 & 127;
-    const int hk = head / p.fa_gq, r = head - hk * p.fa_gq, j = lane & 15;
-    const float *base = p.fa_part + ((size_t)hk * p.fa_ns * 16 + r) * 130;
-    constexpr size_t SS = 16 * 130;
-    // (m, l) of every split and the rows of the first four splits are requested together: one L2 round trip when <= 4 splits are
-    // live (depth <= 512 at 128 cells per split); later groups are only fetched if they hold a live split
-    const float mj = j < p.fa_ns ? __ldcg(base + j * SS + 128) : -INFINITY;
-    const float lj = j < p.fa_ns ? __ldcg(base + j * SS + 129) : 0.0f;
-    float2 o[4][4];
-    auto fetch = [&](int s0) {
-#pragma unroll
-        for (int u = 0; u < 4; u++) {
-            if (s0 + u < p.fa_ns) {
-                const float2 *pp = (const float2 *)(base + (size_t)(s0 + u) * SS + d0);
-#pragma unroll
-                for (int k = 0; k < 4; k++) o[u][k] = __ldcg(pp + k);
-            }
-        }
-    };
-    fetch(0);
-    float M = mj;
-#pragma unroll
-    for (int o2 = 8; o2 > 0; o2 >>= 1) M = fmaxf(M, __shfl_xor_sync(0xffffffffu, M, o2));
-    float L = (j < p.fa_ns && mj != -INFINITY) ? lj * expf(mj - M) : 0.0f;
-#pragma unroll
-    for (int o2 = 8; o2 > 0; o2 >>= 1) L += __shfl_xor_sync(0xffffffffu, L, o2);
-    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    for (int s0 = 0; s0 < p.fa_ns; s0 += 4) {
-        if (s0) {
-            // a group without a live split contributes exact zeros (f = 0): skip its loads (warp-uniform per half: both halves vote)
-            const unsigned livemask = __ballot_sync(0xffffffffu, j >= s0 && j < s0 + 4 && mj != -INFINITY);
-            if (!livemask) continue;
-            fetch(s0);
-        }
-#pragma unroll
-        for (int u = 0; u < 4; u++) {
-            if (s0 + u < p.fa_ns) {
-                const float ms = __shfl_sync(0xffffffffu, mj, (lane & 16) | (s0 + u));
-                const float f = ms == -INFINITY ? 0.0f : expf(ms - M);
-                acc[0] += o[u][0].x * f; acc[1] += o[u][0].y * f; acc[2] += o[u][1].x * f; acc[3] += o[u][1].y * f;
-                acc[4] += o[u][2].x * f; acc[5] += o[u][2].y * f; acc[6] += o[u][3].x * f; acc[7] += o[u][3].y * f;
-            }
-        }
-    }
-    v0 = make_float4(acc[0] / L, acc[1] / L, acc[2] / L, acc[3] / L);
-    v1 = make_float4(acc[4] / L, acc[5] / L, acc[6] / L, acc[7] / L);
-}
-
 // sum over the consumer warps of per-warp partial sums of squares -> 1/rms (rms_norm like glue.cu / the CPU oracle: sum in double)
 // `nact` warps (0 .. nact - 1) hold blocks of the vector: only they meet at the barrier and need the result (the others would add exact zeros)
 __device__ __forceinline__ float bs1_norm_scale(const Bs1Params &p, double *s_red, double s, int warp, int lane, int nact) {
@@ -201,17 +146,6 @@ __device__ __forceinline__ float bs1_norm_scale(const Bs1Params &p, double *s_re
 __device__ __forceinline__ void bs1_prologue(const Bs1Params &p, uint8_t *smem, double *s_red, int warp, int lane) {
     const int nchunk = p.K >> 8, ncw = p.ncw;
     const int cs = p.cs, crank = cs > 1 ? (int)cluster_ctarank() : 0;        // cluster mode: CTA `crank` takes blocks b = cs * j + crank
-    if (p.act_mode == ACT_FA_PART) {             // its own branch: the merge wants the registers the f32 paths keep their vectors in
-        for (int b = warp; b < nchunk; b += ncw) {
-            float4 a0, a1;
-            bs1_load_fa_partials(p, b, lane, a0, a1);
-            const float v[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-            if (p.prof && b == warp) PROFQ(24);
-            bs1_quant_chunk(p, smem, b, lane, v);
-            if (p.prof && b == warp) PROFQ(25);
-        }
-        return;
-    }
     if (nchunk <= 2 * ncw * cs) {
         float4 xa[2][2], xb[2][2];
 #pragma unroll
@@ -534,7 +468,7 @@ int bs1_max_clusters(b200_ctx *ctx, int cs, int threads, size_t smem_bytes) {
 
 // 1 = launched, 0 = not eligible (caller falls through to the general kernel), < 0 = error
 int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_t K, const GemvActDesc &ga, bool w_const,
-                        const GemvPf *pf, int npf, int l2pf, bool *pair, bool dry_run) {
+                        const GemvPf *pf, int npf, int l2pf, bool *pair) {
     const bool want_pair = pair != nullptr;
     if (pair) *pair = false;
     if (!g_bs1_env) {
@@ -548,13 +482,8 @@ int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_
         g_bs1_env = true;
     }
     if (g_bs1_off || nseg < 1 || nseg > GEMV_MAX_SEG || K <= 0 || (K & 255) || K > 65536) return 0;
-    if (ga.mode != ACT_F32 && ga.mode != ACT_F32_NORM && ga.mode != ACT_F32_SWIGLU && ga.mode != ACT_FA_PART) return 0;
-    if (ga.mode == ACT_FA_PART) {
-        // the register-resident prologue only (every llama shape); at launch time the partials must be there
-        if (nseg != 1 || (K & 127) || (K >> 8) > 2 * (g_bs1_warps == 16 ? 15 : 31)) return 0;
-        if (!dry_run && (!ga.fa_part || ga.fa_ns < 2 || ga.fa_ns > 16 || ga.fa_gq < 1 || ((uintptr_t)ga.fa_part & 7))) return 0;
-    }
-    else if (((uintptr_t)ga.x & 15) || (ga.mode != ACT_F32 && ((uintptr_t)ga.x2 & 15))) return 0;
+    if (ga.mode != ACT_F32 && ga.mode != ACT_F32_NORM && ga.mode != ACT_F32_SWIGLU) return 0;
+    if (((uintptr_t)ga.x & 15) || (ga.mode != ACT_F32 && ((uintptr_t)ga.x2 & 15))) return 0;
     int mask = 0;
     for (int s = 0; s < nseg; s++) {
         const int t = segs[s].type;
@@ -565,7 +494,6 @@ int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_
     }
     Bs1Params p = {};
     p.nseg = nseg; p.K = (int)K; p.act_mode = ga.mode; p.x = ga.x; p.x2 = ga.x2; p.eps = ga.eps;
-    p.fa_part = ga.fa_part; p.fa_ns = ga.fa_ns; p.fa_gq = ga.fa_gq;
     p.inv_K = (K & (K - 1)) == 0 ? 1.0 / (double)K : 0.0;
     p.w_const = w_const ? 1 : 0; p.use_pdl = ctx->opt_pdl;
     // shared memory: barriers | s_red | aq64 | aq128 | d | s32 | s16 | ring
@@ -636,7 +564,7 @@ int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_
             budget_pf -= nb < budget_pf ? nb : budget_pf;
         }
     }
-    if (ctx->prof_buf && !dry_run) {     // rotating per-launch slots so consecutive launches can be laid on one timeline
+    if (ctx->prof_buf) {     // rotating per-launch slots so consecutive launches can be laid on one timeline
         p.prof = (unsigned long long *)ctx->prof_buf + (size_t)(ctx->prof_launch % 8) * 296 * 32;
         ctx->prof_launch++;
     }
@@ -666,7 +594,6 @@ int gemv_bs1_try_launch(b200_ctx *ctx, const GemvSegDesc *segs, int nseg, int64_
     for (int s = 0; s < nseg; s++) { p.seg[s].q = (int)(segs[s].N / grid); p.seg[s].rem = (int)(segs[s].N % grid); }
     if (p.pair && (p.cs > 1 || (segs[0].N + grid - 1) / grid > segs[0].N / ctx->sm_count + 1)) { b200_set_error("gemv_bs1: pair-mode row table too small"); return B200_ERR_FAILED; }
     if (pair) *pair = p.pair != 0;
-    if (dry_run) return 1;                  // the launch below would go ahead
     int rc;
     switch (mask) {
         case TB_Q4_K: rc = bs1_launch_t<TB_Q4_K>(ctx, p, (int)grid, smem_bytes); break;

@@ -599,8 +599,6 @@ RopeParams make_rope_params_impl(const int32_t *params) {
 
 }  // namespace
 
-RopeParams make_rope_params(const int32_t *params) { return make_rope_params_impl(params); }
-
 int launch_rope_store(b200_ctx *ctx, const RopeStoreDesc &din) {
     RopeStoreDesc d = din;
     d.use_pdl = ctx->opt_pdl;

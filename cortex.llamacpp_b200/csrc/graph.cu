@@ -9,10 +9,8 @@
 //      replay the captured cudaGraphExec instead of re-launching ~10 kernels per layer.
 #include "common.cuh"
 #include "gemv.h"
-#include "dstep.h"
 #include <string.h>
 #include <algorithm>
-#include <memory>
 
 // A decode step of llama.cpp differs from the previous one ONLY in where the new K/V rows are stored (the CPY destinations are
 // views of the cache at kv_head, llama-graph.cpp:1375-1397).  The reference patches those kernel parameters into its captured
@@ -86,7 +84,7 @@ extern "C" int b200_op_compute(b200_ctx *ctx, const b200_op *op) {
 // A llama layer becomes: [norm+QKV] [rope+store] [flash_attn (+combine)] [wo+residual] [norm+gate|up] [swiglu+down+residual].
 // Intermediates that only lived between the fused ops are never materialised; the matcher proves with a liveness scan
 // over the op list (address ranges, first access after the pattern) that nobody else reads them.
-enum { EX_OP = 0, EX_GEMV = 1, EX_ROPE_STORE = 2, EX_DSTEP = 3 };
+enum { EX_OP = 0, EX_GEMV = 1, EX_ROPE_STORE = 2 };
 static const int g_fuse_debug = getenv("GGML_B200_FUSE_DEBUG") ? atoi(getenv("GGML_B200_FUSE_DEBUG")) : 0;
 struct ExecNode {
     int kind = EX_OP;
@@ -94,11 +92,9 @@ struct ExecNode {
     GemvSegDesc seg[GEMV_MAX_SEG]; int nseg = 0; // EX_GEMV
     int64_t K = 0; GemvActDesc act; int ncols = 0; bool w_const = false;
     GemvPf pf[GEMV_MAX_PF] = {}; int npf = 0;    // L2 look-ahead ranges (weights of the launches that follow)
-    int fa_merge = 0;                            // 1 = FLASH_ATTN op whose KV-split merge the next node (2 = that batch-1 GEMV) can do in its prologue
     int pair = 0;                                // FFN: 1 = gate|up launch (may write silu(gate)*up itself), 2 = the down launch that follows it
     RopeStoreDesc rs;                            // EX_ROPE_STORE
     int kv_slot = -1;                            // index of this node's K destination in the KV pointer table (V = +1)
-    std::shared_ptr<std::vector<DsNode>> ds;     // EX_DSTEP: the run of nodes one persistent decode-step launch executes (dstep.cu)
 };
 
 static bool same_tensor(const b200_tensor &a, const b200_tensor &b) {
@@ -363,61 +359,6 @@ static int match_norm_mm(const b200_op *ops, int n, int i, std::vector<ExecNode>
     return 3;
 }
 
-// Batch-1 decode: maximal runs of nodes the persistent decode-step kernel can execute (fused GEMVs, rope+store followed by its
-// flash attention, plain decode matmuls, row gathers, dense adds) become ONE launch (dstep.cu).  A run needs >= 2 matmuls.
-static void pack_dstep(b200_ctx *ctx, std::vector<ExecNode> &list) {
-    static const int env_skip = getenv("GGML_B200_DEBUG_SKIP") ? atoi(getenv("GGML_B200_DEBUG_SKIP")) : 0;
-    const int dbg_skip = env_skip | ctx->opt_debug_skip;
-    std::vector<ExecNode> out;
-    out.reserve(list.size());
-    size_t i = 0;
-    while (i < list.size()) {
-        std::vector<DsNode> run;
-        size_t j = i;
-        int n_mm = 0;
-        while (j < list.size()) {
-            const ExecNode &e = list[j];
-            DsNode d;
-            if (e.kind == EX_GEMV && dstep_gemv_eligible(ctx, e.seg, e.nseg, e.K, e.act, e.ncols)) {
-                d.kind = DS_GEMV; d.nseg = e.nseg; d.K = e.K; d.act = e.act;
-                for (int s = 0; s < e.nseg; s++) d.seg[s] = e.seg[s];
-                if (!(dbg_skip & 4)) run.push_back(d);
-                n_mm++; j++;
-            } else if (e.kind == EX_ROPE_STORE && j + 1 < list.size() && list[j + 1].kind == EX_OP && list[j + 1].op.op == B200_OP_FLASH_ATTN_EXT &&
-                       dstep_attn_eligible(ctx, e.rs, list[j + 1].op)) {
-                d.kind = DS_ATTN; d.rs = e.rs; d.fa = list[j + 1].op;
-                if (!(dbg_skip & 3)) run.push_back(d);
-                j += 2;
-            } else if (e.kind == EX_OP && e.op.op == B200_OP_MUL_MAT && is_decode_mm(e.op) && e.op.dst.ne[1] == 1 && (e.op.src[0].flags & B200_TENSOR_FLAG_WEIGHT)) {
-                GemvSegDesc sg = seg_of(e.op, (float *)e.op.dst.data, (size_t)e.op.src[0].ne[1], nullptr);
-                GemvActDesc ga = {};
-                ga.mode = ACT_F32; ga.x = (const float *)e.op.src[1].data; ga.x_stride = e.op.src[1].nb[1];
-                if (!dstep_gemv_eligible(ctx, &sg, 1, e.op.src[0].ne[0], ga, 1)) break;
-                d.kind = DS_GEMV; d.nseg = 1; d.K = e.op.src[0].ne[0]; d.act = ga; d.seg[0] = sg;
-                if (!(dbg_skip & 4)) run.push_back(d);
-                n_mm++; j++;
-            } else if (e.kind == EX_OP && (e.op.op == B200_OP_GET_ROWS || e.op.op == B200_OP_ADD) && dstep_copy_eligible(e.op) && !run.empty()) {
-                d.kind = DS_COPY; d.cp = e.op;
-                run.push_back(d);
-                j++;
-            } else break;
-        }
-        // trailing gathers / adds without a consumer inside the run stay ordinary launches
-        while (j > i && !run.empty() && run.back().kind == DS_COPY) { run.pop_back(); j--; }
-        if (n_mm >= 2 && !run.empty()) {
-            ExecNode m;
-            m.kind = EX_DSTEP;
-            m.ds = std::make_shared<std::vector<DsNode>>(std::move(run));
-            out.push_back(m);
-            i = j;
-        } else {
-            out.push_back(list[i]);
-            i++;
-        }
-    }
-    list.swap(out);
-}
-
 // returns the list actually executed
 static int fuse(b200_ctx *ctx, const b200_op *ops, int n, std::vector<ExecNode> &out) {
     out.clear();
@@ -510,45 +451,6 @@ static int fuse(b200_ctx *ctx, const b200_op *ops, int n, std::vector<ExecNode> 
         size_t k = j + 1;
         if (k < out.size() && gemv_like(out[k])) { add_ranges(e, out[k]); covered[k] = 1; }
     }
-    // split merge in the consumer: a batch-1 FLASH_ATTN node directly followed by the fused output-projection GEMV that reads its
-    // result as plain f32 activations.  The attention output must be dead afterwards: scanning the nodes that follow, the first touch of
-    // its range has to be a full overwrite (ggml-alloc reuses the buffer), not a read.
-    if (layer_fusion) {
-        auto rng = [](const void *ptr, size_t bytes, uintptr_t &lo, uintptr_t &hi) { lo = (uintptr_t)ptr; hi = lo + bytes; };
-        for (size_t i = 0; i + 1 < out.size(); i++) {
-            ExecNode &fa = out[i], &mm = out[i + 1];
-            if (fa.kind != EX_OP || fa.op.op != B200_OP_FLASH_ATTN_EXT || mm.kind != EX_GEMV) continue;
-            const b200_tensor &q = fa.op.src[0], &d = fa.op.dst;
-            if (q.ne[1] != 1 || q.ne[0] != 128 || mm.ncols != 1 || mm.nseg != 1 || mm.act.mode != ACT_F32 || mm.act.x != (const float *)d.data ||
-                mm.K != q.ne[0] * q.ne[2] || mm.seg[0].expert_id) continue;
-            uintptr_t lo, hi;
-            rng(d.data, (size_t)mm.K * 4, lo, hi);
-            auto touches = [&](const void *ptr, size_t bytes) { uintptr_t a, b; rng(ptr, bytes, a, b); return ptr && a < hi && lo < b; };
-            auto covers = [&](const void *ptr, size_t bytes) { uintptr_t a, b; rng(ptr, bytes, a, b); return ptr && a <= lo && hi <= b; };
-            if (touches(mm.seg[0].residual, (size_t)mm.seg[0].N * 4)) continue;
-            bool dead = false, live = false;
-            for (size_t j = i + 2; j < out.size() && !dead && !live; j++) {
-                const ExecNode &e = out[j];
-                if (e.kind == EX_OP) {
-                    for (int t = 0; t < e.op.n_src && !live; t++) { uintptr_t a, b; tensor_range(e.op.src[t], a, b); live = e.op.src[t].data && a < hi && lo < b; }
-                    if (!live) { uintptr_t a, b; tensor_range(e.op.dst, a, b); if (a <= lo && hi <= b) dead = true; else if (a < hi && lo < b) live = true; }
-                } else if (e.kind == EX_GEMV) {
-                    const size_t xb = (size_t)e.K * 4;
-                    live = touches(e.act.x, xb) || (e.act.mode != ACT_F32 && touches(e.act.x2, xb));
-                    for (int t = 0; t < e.nseg && !live; t++) live = touches(e.seg[t].residual, (size_t)e.seg[t].N * 4);
-                    for (int t = 0; t < e.nseg && !live && !dead; t++) { if (covers(e.seg[t].dst, (size_t)e.seg[t].N * 4)) dead = true; else if (touches(e.seg[t].dst, (size_t)e.seg[t].N * 4)) live = true; }
-                } else if (e.kind == EX_ROPE_STORE) {    // reads q, k, v of the ubatch; writes the roped q (a write that does not cover the whole range counts as a touch)
-                    const RopeStoreDesc &r = e.rs;
-                    const size_t qb = (size_t)r.T * r.H * r.D * 4, kb = (size_t)r.T * r.Hkv * r.D * 4;
-                    live = touches(r.q, qb) || touches(r.k, kb) || touches(r.v, kb);
-                    if (!live) { if (covers(r.q_out, qb)) dead = true; else if (touches(r.q_out, qb)) live = true; }
-                } else live = true;                      // decode-step nodes: not analysed, keep the merged output
-            }
-            if (live) continue;                          // (never touched again also counts as dead)
-            fa.fa_merge = 1; mm.fa_merge = 2;
-        }
-    }
-    if (layer_fusion && ctx->opt_dstep) pack_dstep(ctx, out);
     return B200_OK;
 }
 
@@ -565,27 +467,7 @@ static int run_list(b200_ctx *ctx, const std::vector<ExecNode> &list) {
             if ((dbg_skip & 4) && e.kind == EX_GEMV) continue;
             if ((dbg_skip & 8) && e.kind == EX_OP && e.op.op == B200_OP_ALLREDUCE) continue;
         }
-        if (e.kind == EX_DSTEP) {
-            DsProgram *prog = nullptr;
-            rc = dstep_prepare(ctx, *e.ds, &prog);           // cached by content: a hit (no upload) once prepare_dstep() has seen this list
-            if (!rc) rc = dstep_launch(ctx, prog);
-        }
-        else if (e.kind == EX_OP && e.fa_merge == 1 && ctx->opt_fa_merge_in_wo && (&e + 1) < list.data() + list.size() && (&e + 1)->fa_merge == 2 && !dbg_skip) {
-            // would the batch-1 GEMV take the output projection with the split merge in its prologue?  (dry run: no launch)
-            const ExecNode &mm = *(&e + 1);
-            GemvActDesc a = mm.act; a.mode = ACT_FA_PART;
-            const bool can = gemv_bs1_try_launch(ctx, mm.seg, mm.nseg, mm.K, a, mm.w_const, nullptr, 0, 0, nullptr, true) == 1;
-            ctx->fa_part_ns = 0; ctx->fa_part = nullptr;
-            ctx->fa_skip_combine = can;
-            rc = dispatch(ctx, &e.op);
-            ctx->fa_skip_combine = false;
-        }
-        else if (e.kind == EX_GEMV && e.fa_merge == 2 && ctx->fa_part_ns > 1) {
-            GemvActDesc a = e.act; a.mode = ACT_FA_PART; a.fa_part = ctx->fa_part; a.fa_ns = ctx->fa_part_ns; a.fa_gq = ctx->fa_part_gq;
-            ctx->fa_part_ns = 0;
-            rc = gemv_launch(ctx, e.seg, e.nseg, e.K, a, e.ncols, e.w_const, e.pf, e.npf);
-        }
-        else if (e.kind == EX_GEMV) {
+        if (e.kind == EX_GEMV) {
             if (e.pair == 1 && ctx->opt_ffn_pair) rc = gemv_launch(ctx, e.seg, e.nseg, e.K, e.act, e.ncols, e.w_const, e.pf, e.npf, &pair_done);
             else if (e.pair == 2 && pair_done) {          // the gate|up launch left h = silu(gate) * up in the gate scratch: plain f32 activations
                 GemvActDesc a = e.act; a.mode = ACT_F32; a.x2 = nullptr;
@@ -608,15 +490,12 @@ static bool is_kv_store(const b200_op &o) {
     return d.ne[1] == 1 && d.ne[2] == 1 && d.ne[3] == 1 && !(d.flags & B200_TENSOR_FLAG_WEIGHT);
 }
 
-// point every fused rope+store node at its slots of the entry's device table; false if a KV store is not inside such a node
-// every rope+store descriptor of a list: plain EX_ROPE_STORE nodes and the attention nodes inside decode-step runs
+// every rope+store descriptor of a list
 static void collect_rope_stores(std::vector<ExecNode> &list, std::vector<RopeStoreDesc *> &out) {
     out.clear();
-    for (ExecNode &x : list) {
-        if (x.kind == EX_ROPE_STORE) out.push_back(&x.rs);
-        else if (x.kind == EX_DSTEP) for (DsNode &d : *x.ds) if (d.kind == DS_ATTN) out.push_back(&d.rs);
-    }
+    for (ExecNode &x : list) if (x.kind == EX_ROPE_STORE) out.push_back(&x.rs);
 }
+// point every fused rope+store node at its slots of the entry's device table; false if a KV store is not inside such a node
 static bool bind_kv_table(GraphCacheEntry &e, const b200_op *ops, std::vector<ExecNode> &list, bool assign) {
     e.node_kv.clear();
     size_t covered = 0;
@@ -642,41 +521,6 @@ static void unbind_kv_table(std::vector<ExecNode> &list) {
     collect_rope_stores(list, rss);
     for (RopeStoreDesc *rs : rss) rs->k_dst_ind = rs->v_dst_ind = nullptr;
 }
-// Eagerly run lists: the decode-step programs are cached by content, and the KV-store destinations change every token.  Route
-// them through a context-owned device table (refreshed here, stream-ordered) so that the program stays the same from step to step.
-static int bind_eager_kv(b200_ctx *ctx, std::vector<ExecNode> &list) {
-    bool any = false;
-    for (ExecNode &x : list) any |= x.kind == EX_DSTEP;
-    if (!any) return B200_OK;
-    std::vector<RopeStoreDesc *> rss;
-    collect_rope_stores(list, rss);
-    if (rss.empty() || rss.size() > 512) return B200_OK;
-    if (!ctx->eager_kv_table && cudaMalloc((void **)&ctx->eager_kv_table, 2 * 512 * sizeof(void *)) != cudaSuccess) { cudaGetLastError(); ctx->eager_kv_table = nullptr; return B200_OK; }
-    void *host[2 * 512];
-    for (size_t j = 0; j < rss.size(); j++) {
-        host[2 * j] = rss[j]->k_dst; host[2 * j + 1] = rss[j]->v_dst;
-        rss[j]->k_dst_ind = (void *const *)(ctx->eager_kv_table + 2 * j); rss[j]->v_dst_ind = (void *const *)(ctx->eager_kv_table + 2 * j + 1);
-    }
-    CUDA_TRY(cudaMemcpyAsync(ctx->eager_kv_table, host, 2 * rss.size() * sizeof(void *), cudaMemcpyHostToDevice, ctx->stream));
-    return B200_OK;
-}
-// upload (or find) the decode-step programs of a list before any launch -- in particular before stream capture begins
-static int prepare_dstep(b200_ctx *ctx, std::vector<ExecNode> &list) {
-    for (ExecNode &x : list) {
-        if (x.kind != EX_DSTEP) continue;
-        DsProgram *prog = nullptr;
-        int rc = dstep_prepare(ctx, *x.ds, &prog);
-        if (rc) return rc;
-    }
-    return B200_OK;
-}
-static int run_eager(b200_ctx *ctx, std::vector<ExecNode> &list) {
-    int rc = bind_eager_kv(ctx, list);
-    if (!rc) rc = prepare_dstep(ctx, list);
-    if (!rc) rc = run_list(ctx, list);
-    return rc;
-}
-
 static int upload_kv_table(b200_ctx *ctx, const GraphCacheEntry &e, const b200_op *ops) {
     if (e.node_kv.empty()) return B200_OK;
     void *host[2 * 512];
@@ -742,20 +586,20 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
     if (ctx->opt_fusion) { int frc = fuse(ctx, ops, n_ops, list); if (frc) return frc; }
     else { list.resize(n_ops); for (int i = 0; i < n_ops; i++) list[i].op = ops[i]; }
 
-    if (!ctx->opt_cuda_graphs || n_ops < 8) return run_eager(ctx, list);
+    if (!ctx->opt_cuda_graphs || n_ops < 8) return run_list(ctx, list);
     for (int i = 0; i < n_ops; i++)            // row-split matmuls fork to other devices' streams: launched eagerly
-        if (ops[i].op == B200_OP_MUL_MAT && (ops[i].src[0].flags & B200_TENSOR_FLAG_SPLIT)) return run_eager(ctx, list);
+        if (ops[i].op == B200_OP_MUL_MAT && (ops[i].src[0].flags & B200_TENSOR_FLAG_SPLIT)) return run_list(ctx, list);
 
     // only decode-sized steps repeat (a prompt ubatch is seen once, and capturing its ~1000 big launches costs more than it saves)
     {
         bool decode_like = false;
         for (const ExecNode &x : list) {
-            decode_like |= x.kind == EX_GEMV || x.kind == EX_DSTEP;
+            decode_like |= x.kind == EX_GEMV;
             // a continuous-batching step (<= 32 token columns) repeats like a decode step
             decode_like |= x.kind == EX_OP && x.op.op == B200_OP_MUL_MAT && x.op.src[1].ne[1] <= 32 && (x.op.src[0].flags & B200_TENSOR_FLAG_WEIGHT) &&
                            b200_type_is_quant(x.op.src[0].type);
         }
-        if (!decode_like && ctx->opt_fusion >= 2) return run_eager(ctx, list);
+        if (!decode_like && ctx->opt_fusion >= 2) return run_list(ctx, list);
     }
     // ---- CUDA graph replay keyed on the op list modulo the KV-store destinations ----
     if (!ctx->graph_cache) ctx->graph_cache = new GraphCache();
@@ -787,12 +631,6 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
             if (e.indirect) { int rc = upload_kv_table(ctx, e, ops); if (rc) return rc; }
             else { e.kv_ptrs.clear(); for (int idx : kv_idx) e.kv_ptrs.push_back(ops[idx].dst.data); unbind_kv_table(list); }
         }
-        {   // decode-step programs are uploaded before the capture starts; if that grew a scratch area the graph cache (and `e`) is gone
-            const int64_t gen = ctx->scratch_gen;
-            int prc = prepare_dstep(ctx, list);
-            if (prc) return prc;
-            if (gen != ctx->scratch_gen) { unbind_kv_table(list); return run_eager(ctx, list); }
-        }
         cudaGraph_t g = nullptr;
         ctx->capturing = true;
         CUDA_TRY(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
@@ -803,12 +641,12 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
             cudaGetLastError();
             if (g) cudaGraphDestroy(g);
             unbind_kv_table(list);
-            return run_eager(ctx, list);          // fall back to eager launches
+            return run_list(ctx, list);          // fall back to eager launches
         }
         if (cudaGraphInstantiate(&e.exec, g, 0) != cudaSuccess) {
             cudaGetLastError(); e.exec = nullptr; cudaGraphDestroy(g);
             unbind_kv_table(list);
-            return run_eager(ctx, list);
+            return run_list(ctx, list);
         }
         cudaGraphDestroy(g);
         CUDA_TRY(cudaGraphLaunch(e.exec, ctx->stream));
@@ -834,9 +672,8 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
     }
     if (gdebug) {
         int ng = 0, nr = 0;
-        int nd = 0;
-        for (const ExecNode &x : list) { ng += x.kind == EX_GEMV; nr += x.kind == EX_ROPE_STORE; nd += x.kind == EX_DSTEP; }
-        fprintf(stderr, "[b200 graph] new list: %d ops -> %zu nodes (%d fused gemv, %d rope+store, %d decode-step runs), %zu kv stores; op ids:", n_ops, list.size(), ng, nr, nd, kv_idx.size());
+        for (const ExecNode &x : list) { ng += x.kind == EX_GEMV; nr += x.kind == EX_ROPE_STORE; }
+        fprintf(stderr, "[b200 graph] new list: %d ops -> %zu nodes (%d fused gemv, %d rope+store), %zu kv stores; op ids:", n_ops, list.size(), ng, nr, kv_idx.size());
         for (int i = 0; i < n_ops && i < 64; i++) fprintf(stderr, " %d", ops[i].op);
         fprintf(stderr, "\n");
     }
@@ -846,5 +683,5 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
     for (int idx : kv_idx) ne.kv_ptrs.push_back(ops[idx].dst.data);
     ne.indirect = !kv_idx.empty() && bind_kv_table(ne, ops, list, false);
     gc.entries.push_back(std::move(ne));
-    return run_eager(ctx, list);
+    return run_list(ctx, list);
 }

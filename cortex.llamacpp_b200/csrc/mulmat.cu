@@ -6,8 +6,8 @@
 // 16-bit float weights) and every dst element is one dot product.
 //   quantised W, M <= 4      : streaming GEMV, activation quantisation in its prologue (gemv.cu, gemv_bs1.cu)
 //   quantised W, 5 <= M <= 32: quantise (quant.cu) + small-batch mma.sync kernel (gemv_mma.cu)
-//   quantised W, M > 32      : prompt-batch GEMM on mma.sync (gemm_mma.cu, all five formats); GGML_B200_PREFER_TCGEN05=1: tcgen05 int8 GEMM
-//                              (gemm_i8.cu, K-quants); shapes neither takes (N % 128, K % 256): GEMV in column chunks
+//   quantised W, M > 32      : K-quants: tcgen05 kind::f16 GEMM (gemm_tc.cu); other formats: prompt-batch GEMM on mma.sync (gemm_mma.cu);
+//                              shapes neither takes (N % 128, K % 256): GEMV in column chunks
 //   row-split W (B200_TENSOR_FLAG_SPLIT): every shard's GPU at once (op_mul_mat_split)
 //   F32/F16/BF16 W           : warp-per-row float kernel below (MoE router, small test shapes)
 //   cpu_exact mode           : exact.cu (the reference AVX2 build's summation order)
@@ -16,7 +16,6 @@
 #include "common.cuh"
 #include <algorithm>
 #include <cuda_bf16.h>
-#include "gemm_i8.h"
 #include "gemm_tc.h"
 
 int gemv_max_cols(const b200_ctx *ctx, int type, size_t rb, int64_t K);
@@ -259,12 +258,9 @@ int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
     // continuous-batching decode (9..32 columns): weight-streaming mma.sync kernel (gemv_mma.cu); q4_0 / q8_0, which the tcgen05
     // GEMM does not decode, go through it in chunks of 32 columns at any batch size
     static const int64_t mma_max_m = getenv("GGML_B200_MMA_MAX_M") ? atoi(getenv("GGML_B200_MMA_MAX_M")) : 32;
-    // prompt batches: the mma.sync tile GEMM (gemm_mma.cu, all five formats); GGML_B200_PREFER_TCGEN05=1 sends K-quants to the tcgen05
-    // GEMM instead (gemm_i8.cu: correct, but its CUDA-core stages keep it below the mma.sync kernel -- DESIGN.md 8)
-    static const int prefer_tc = getenv("GGML_B200_PREFER_TCGEN05") ? atoi(getenv("GGML_B200_PREFER_TCGEN05")) : 0;
     // K-quants from tc_min_m token columns up: the tcgen05 kind::f16 GEMM (gemm_tc.cu: exact-integer f16 operands, min term on the tensor core)
     static const int64_t tc_min_m = getenv("GGML_B200_TC_MIN_M") ? atoi(getenv("GGML_B200_TC_MIN_M")) : 33;
-    if (M >= tc_min_m && !prefer_tc && x.nb[0] == 4 && gemm_tc_supported(w.type, N, K, M) && !((uintptr_t)w.data & 15) && !(w.nb[2] & 15) && !(w.nb[3] & 15)) {
+    if (M >= tc_min_m && x.nb[0] == 4 && gemm_tc_supported(w.type, N, K, M) && !((uintptr_t)w.data & 15) && !(w.nb[2] & 15) && !(w.nb[3] & 15)) {
         for (int64_t i3 = 0; i3 < x.ne[3]; i3++)
             for (int64_t i2 = 0; i2 < x.ne[2]; i2++) {
                 const int64_t w2 = i2 / (x.ne[2] / w.ne[2]), w3 = i3 / (x.ne[3] / w.ne[3]);
@@ -276,7 +272,8 @@ int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
             }
         return B200_OK;
     }
-    if (M > mma_max_m && gemm_mma_supported(w.type, N, K, M) && !(prefer_tc && gemm_i8_supported(w.type, N, K, M))) {
+    // prompt batches the tcgen05 GEMM does not take: the mma.sync tile GEMM (gemm_mma.cu, all five formats)
+    if (M > mma_max_m && gemm_mma_supported(w.type, N, K, M)) {
         for (int64_t i3 = 0; i3 < x.ne[3]; i3++)
             for (int64_t i2 = 0; i2 < x.ne[2]; i2++) {
                 const int64_t w2 = i2 / (x.ne[2] / w.ne[2]), w3 = i3 / (x.ne[3] / w.ne[3]);
@@ -288,7 +285,7 @@ int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
             }
         return B200_OK;
     }
-    if (gemv_mma_supported(w.type, N, K, M) && (M <= mma_max_m || !gemm_i8_supported(w.type, N, K, M))) {
+    if (gemv_mma_supported(w.type, N, K, M)) {
         uint8_t *act = (uint8_t *)ctx->get_scratch(SCRATCH_ACT, L.col_bytes * (size_t)M);
         if (!act) return B200_ERR_ALLOC;
         for (int64_t i3 = 0; i3 < x.ne[3]; i3++)
@@ -301,19 +298,6 @@ int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
                 for (int64_t c0 = 0; c0 < M && !rc; c0 += 32)
                     rc = launch_gemv_mma(ctx, w.type, wp, rb, N, K, act + (size_t)c0 * L.col_bytes, (int)(M - c0 < 32 ? M - c0 : 32),
                                          dp + (size_t)c0 * (d.nb[1] / 4), d.nb[1] / 4, M <= 32, w_const);
-                if (rc) return rc;
-            }
-        return B200_OK;
-    }
-    // prefill: K-quant weights go to the tensor cores (tcgen05 int8 GEMM with the CPU's exact q8_K integer stage)
-    if (gemm_i8_supported(w.type, N, K, M) && x.nb[0] == 4) {
-        for (int64_t i3 = 0; i3 < x.ne[3]; i3++)
-            for (int64_t i2 = 0; i2 < x.ne[2]; i2++) {
-                const int64_t w2 = i2 / (x.ne[2] / w.ne[2]), w3 = i3 / (x.ne[3] / w.ne[3]);
-                const uint8_t *wp = (const uint8_t *)w.data + w2 * w.nb[2] + w3 * w.nb[3];
-                const float *xp = (const float *)((const char *)x.data + i2 * x.nb[2] + i3 * x.nb[3]);
-                float *dp = (float *)((char *)d.data + i2 * d.nb[2] + i3 * d.nb[3]);
-                int rc = gemm_i8_run(ctx, w.type, wp, rb, N, K, xp, x.nb[1], M, dp, d.nb[1] / 4);
                 if (rc) return rc;
             }
         return B200_OK;
@@ -430,8 +414,7 @@ int op_mul_mat_id(b200_ctx *ctx, const b200_op *op) {
         if (npairs >= 32 * E && gemm_mma_supported(as.type, N, K, 128)) {
             g.max_chunks = (int)std::min<int64_t>(npairs, npairs / 128 + E);
             // K-quants: the tcgen05 kind::f16 GEMM in grouped mode (gemm_tc.cu); Q4_0 / Q8_0: the mma.sync tile GEMM
-            static const int prefer_i8 = getenv("GGML_B200_PREFER_TCGEN05") ? atoi(getenv("GGML_B200_PREFER_TCGEN05")) : 0;
-            if (!prefer_i8 && gemm_tc_supported(as.type, N, K, 128) && !(((uintptr_t)as.data | as.nb[2]) & 15))
+            if (gemm_tc_supported(as.type, N, K, 128) && !(((uintptr_t)as.data | as.nb[2]) & 15))
                 return gemm_tc_run_grouped(ctx, as.type, (const uint8_t *)as.data, rb, N, K, (const float *)b.data, b.ne[1] == 1 ? b.nb[2] : b.nb[1], g, (float *)d.data);
             return gemm_mma_run_grouped(ctx, as.type, (const uint8_t *)as.data, rb, N, K, (const float *)b.data, b.ne[1] == 1 ? b.nb[2] : b.nb[1], g, (float *)d.data);
         }

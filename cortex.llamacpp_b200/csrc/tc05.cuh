@@ -1,5 +1,5 @@
-// tc05.cuh -- tcgen05 / TMEM / UMMA shared-memory descriptor primitives (inline PTX) shared by the tensor-core GEMMs
-// (gemm_i8.cu: kind::i8 with hi/lo operand tiles, gemm_tc.cu: kind::f16 with exact-integer f16 operands).
+// tc05.cuh -- tcgen05 / TMEM / UMMA shared-memory descriptor primitives (inline PTX) shared by the tensor-core kernels
+// (gemm_tc.cu: kind::f16 GEMM with exact-integer f16 operands, fattn_tc.cu: flash attention).
 #pragma once
 #include "common.cuh"
 

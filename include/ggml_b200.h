@@ -154,9 +154,9 @@ B200_API int         b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n
 B200_API int         b200_op_compute(b200_ctx *ctx, const b200_op *op);   /* single op, no fusion */
 B200_API int64_t     b200_kernel_launches(const b200_ctx *ctx);       /* kernels launched by this ctx so far (bench: gpu_launches) */
 /* keys: "cuda_graphs", "fusion" (0 off, 1 two-op, 2 + llama layer fusions), "pdl", "cpu_exact" (parity mode: the reference CPU
- * backend's summation order), "l2_prefetch" (0 off / 1 / 2), "ffn_pair" (gate|up GEMV writes silu(gate)*up; default 1),
- * "fa_merge_in_wo" (output projection merges the flash-attention KV splits; default 0), "dstep" (persistent decode-step kernel;
- * default 0), "debug_skip" (timing experiments only).  Changing one drops the captured CUDA graphs. */
+ * backend's summation order; "fa_exact" is an alias), "l2_prefetch" (0 off / 1 / 2), "ffn_pair" (gate|up GEMV writes
+ * silu(gate)*up; default 1), "debug_skip" (timing experiments only).  Changing one drops the captured CUDA graphs.
+ * Any other key returns B200_ERR_UNSUPPORTED. */
 B200_API int         b200_set_option(b200_ctx *ctx, const char *key, int value);
 
 /* ---- tensor parallelism: one process (and one b200_ctx) per GPU ------------------------------

@@ -1,8 +1,8 @@
 """GPU parity of the prompt-batch GEMMs against the oracle's mul_mat (ggml_compute_forward_mul_mat with q8_K / q8_0 activations):
 the tcgen05 kind::f16 GEMM (gemm_tc.cu: K-quants, the default for more than 32 token columns; its 32- and 64-token tiles and split-K
 are exercised in a subprocess with GGML_B200_TC_MIN_M=5), the mma.sync tile GEMM (gemm_mma.cu: all five formats; the default for
-Q4_0 / Q8_0, for K-quants selected with GGML_B200_NO_GEMM_TC=1) and the round-1 tcgen05 int8 GEMM (gemm_i8.cu,
-GGML_B200_PREFER_TCGEN05=1).  The integer stage is the CPU's exactly, so the results agree to f32 summation order: 3e-6 relative."""
+Q4_0 / Q8_0, for K-quants selected with GGML_B200_NO_GEMM_TC=1).  The integer stage is the CPU's exactly, so the results agree
+to f32 summation order: 3e-6 relative."""
 import os
 import subprocess
 import sys
@@ -61,27 +61,6 @@ def test_gemm_mma_whole_matrix_and_determinism(b200, ctx, t):
     want = R.orc_mul_mat(t, W, x, N, K)
     assert np.abs(got - want).max() <= 3e-6 * np.abs(want).max()
     assert np.array_equal(got, gpu_mul_mat(b200, ctx, t, W, x, N, K))
-
-
-def test_tcgen05_gemm_still_green_when_selected():
-    """GGML_B200_PREFER_TCGEN05=1 routes K-quant prompt batches to the tcgen05 kind::i8 GEMM (read once per process)"""
-    env = dict(os.environ, GGML_B200_PREFER_TCGEN05="1")
-    code = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-            "import numpy as np, reflib as R\n"
-            "from conftest import load_package\n"
-            "from util import dev_bytes, rand_quant_rows, to_dev\n"
-            "b200 = load_package(); ctx = b200.Context(0)\n"
-            "for t in (R.Q4_K, R.Q5_K, R.Q6_K):\n"
-            "    rng = np.random.default_rng(t); N, K, M = 256, 1024, 130\n"
-            "    W = rand_quant_rows(t, N, K, rng); x = rng.standard_normal((M, K)).astype(np.float32)\n"
-            "    Wd = dev_bytes(W.size + 256, 0); Wd[:W.size] = to_dev(W); xd = to_dev(x); out = dev_bytes(M * N * 4, 0xFF)\n"
-            "    op = b200.make_op(b200.OP_MUL_MAT, b200.tensor(out.data_ptr(), b200.F32, [N, M]), [b200.tensor(Wd.data_ptr(), t, [K, N], flags=1), b200.tensor(xd.data_ptr(), b200.F32, [K, M])])\n"
-            "    l0 = ctx.launches(); ctx.compute_op(op); ctx.sync()\n"
-            "    got = out.cpu().numpy().view(np.float32).reshape(M, N); want = R.orc_mul_mat(t, W, x, N, K)\n"
-            "    assert np.abs(got - want).max() <= 3e-6 * np.abs(want).max(), t\n"
-            "print('TCGEN05 OK')\n") % (os.path.dirname(os.path.abspath(__file__)), os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0 and "TCGEN05 OK" in p.stdout, p.stdout[-500:] + p.stderr[-1500:]
 
 
 def _run_gemm_cases(env_extra, cases, tag):

@@ -201,43 +201,6 @@ def test_ffn_pair_epilogue_bit_identical(b200, ctx, model, ftype):
         assert np.array_equal(ref, v), k
 
 
-@pytest.mark.parametrize("model,kv,n_kv,depth", [("mid-d128", "f16", 256, 5), ("mid-d128", "q8_0", 1024, 700), ("tiny-d128", "f16", 2048, 1500), ("mid-d128", "q4_0", 768, 512)])
-def test_fa_split_merge_in_output_projection_bit_identical(b200, ctx, model, kv, n_kv, depth):
-    """option fa_merge_in_wo (opt-in: correct but measured slower, DESIGN.md 8): at batch 1 the flash-attention launch leaves its KV-split partials unmerged and the fused output-projection
-    GEMV merges them in its activation prologue (gemv_bs1.cu bs1_load_fa_partials: the combine kernel's arithmetic in the same order) --
-    one launch less per layer, logits bit-identical, eager and under CUDA-graph replay"""
-    import torch
-    from __graft_entry__ import load_llama_graph
-    lg = load_llama_graph()
-    g = lg.LlamaGraph(b200, model=model, ftype="q4_k_m", kv=kv, n_ctx=n_kv, max_tokens=1)
-    g.fill_cache(depth)
-    rng = np.random.default_rng(13)
-    emb, pos, mask = g.set_inputs_host(1, depth, n_kv, rng)
-    g.inp_embd[:g.E] = torch.from_numpy(emb.reshape(-1)).cuda()
-    g.pos[:1] = torch.from_numpy(pos).cuda()
-    g.mask_f32[:mask.size] = torch.from_numpy(mask.reshape(-1)).cuda()
-    torch.cuda.synchronize()
-    ops = g.build(1, depth, n_kv)
-    ctx.set_option("fusion", 2); ctx.set_option("pdl", 1)
-    outs, launches = {}, {}
-    for graphs in (0, 1):
-        ctx.set_option("cuda_graphs", graphs)
-        for merge in (0, 1):
-            ctx.set_option("fa_merge_in_wo", merge)
-            for it in range(3):
-                g.logits.zero_(); torch.cuda.synchronize()
-                n0 = ctx.launches()
-                ctx.compute(ops); ctx.sync()
-                if it == 0: launches[(graphs, merge)] = ctx.launches() - n0
-            outs[(graphs, merge)] = g.logits[:g.V].cpu().numpy().copy()
-    ctx.set_option("fa_merge_in_wo", 0); ctx.set_option("pdl", 0); ctx.set_option("cuda_graphs", 0)
-    ref = outs[(0, 0)]
-    assert np.isfinite(ref).all() and np.abs(ref).max() > 0
-    for k, v in outs.items():
-        assert np.array_equal(ref, v), k
-    assert launches[(0, 1)] == launches[(0, 0)] - len(g.layers), launches       # the combine launch of every layer is gone
-
-
 def test_l2_lookahead_modes_do_not_change_results(b200, ctx):
     """option l2_prefetch (0 off, 1 next matmul with the first copies, 2 following launches' ranges after the launch's own copies, across
     the attention chain): a pure L2 hint -- logits bit-identical in every mode (gemv_bs1.cu bs1_l2_lookahead, graph.cu look-ahead pass)"""
@@ -345,50 +308,3 @@ def test_graph_replay_survives_scratch_growth(b200, ctx):
         ctx.compute(ops_small); ctx.sync()
         assert np.array_equal(g.logits[:g.V].cpu().numpy(), eager)
     ctx.set_option("pdl", 0); ctx.set_option("cuda_graphs", 0)
-
-
-@pytest.mark.parametrize("model,ftype,kv", [("tiny-d128", "q4_k_m", "f16"), ("tiny-d128", "q4_k_m", "q8_0"), ("tiny-d128", "q5_k_m", "q4_0"),
-                                            ("mid-d128", "q4_k_m", "f16"), ("mid-d128", "q5_k_m", "q8_0")])
-def test_decode_step_kernel_vs_per_launch_path(b200, ctx, model, ftype, kv):
-    """option dstep: a batch-1 decode step as ONE persistent kernel (dstep.cu) against the per-launch fused path it replaces, on
-    the same cache contents: the GEMV phases use the same block decoders (identical integers) and the attention phase the same
-    arithmetic, so every single step must agree to float-summation-order noise; the whole loop stays inside the fast-mode envelope
-    of the oracle; and the step must really be one decode-step launch (+ the mask conversion)."""
-    import torch
-    import llama_forward as OF
-    from __graft_entry__ import load_llama_graph
-    lg = load_llama_graph()
-    g = lg.LlamaGraph(b200, model=model, ftype=ftype, kv=kv, n_ctx=512, max_tokens=4)
-    ctx.set_option("fusion", 2); ctx.set_option("cuda_graphs", 0); ctx.set_option("pdl", 1)
-    rng = np.random.default_rng(11)
-    g.fill_cache(300)
-    caches = None
-    worst_pair, worst_orc = 0.0, 0.0
-    try:
-        for step in range(6):
-            kv_head, n_kv = 300 + step, 512
-            emb, pos, mask = g.set_inputs_host(1, kv_head, n_kv, rng)
-            g.inp_embd[:g.E] = torch.from_numpy(emb.reshape(-1)).cuda()
-            g.pos[:1] = torch.from_numpy(pos).cuda()
-            g.mask_f32[:mask.size] = torch.from_numpy(mask.reshape(-1)).cuda()
-            torch.cuda.synchronize()
-            want, caches = OF.forward(g, emb, pos, mask, kv_head, n_kv, caches=caches)
-            ops = g.build(1, kv_head, n_kv)
-            outs, launches = {}, {}
-            for d in (0, 1):                      # the per-launch run writes the same K/V cell first; the decode-step run overwrites it with equal bytes
-                ctx.set_option("dstep", d)
-                g.logits.zero_(); torch.cuda.synchronize()
-                n0 = ctx.launches()
-                ctx.compute(ops); ctx.sync()
-                launches[d] = ctx.launches() - n0
-                outs[d] = g.logits[:g.V].cpu().numpy().copy()
-            assert np.isfinite(outs[1]).all()
-            pair = float(np.abs(outs[0] - outs[1]).max() / np.abs(outs[0]).max())
-            orc = float(np.abs(outs[1] - want[0]).max() / np.abs(want[0]).max())
-            worst_pair, worst_orc = max(worst_pair, pair), max(worst_orc, orc)
-            assert launches[1] <= 2 < launches[0], launches
-            assert orc <= FAST_MODE_BOUND, (step, orc)
-            assert pair <= FAST_MODE_BOUND, (step, pair)
-        print("dstep %s %s %s: worst vs per-launch path %.3g, vs oracle %.3g" % (model, ftype, kv, worst_pair, worst_orc))
-    finally:
-        ctx.set_option("dstep", 1); ctx.set_option("pdl", 0)

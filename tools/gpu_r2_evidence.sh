@@ -11,6 +11,5 @@ python tools/summarize_launches.py gpurun_out/r2_launches_bench.csv > gpurun_out
 timeout 1200 ncu --metrics dram__bytes_read.sum,dram__bytes_write.sum,gpu__time_duration.sum --clock-control none -k regex:gemv_bs1 -s 516 -c 129 --csv --log-file gpurun_out/r2_ncu_bs1_traffic.csv python bench.py --steps 2 --warmup 3 --no-cpu --no-batch --graphs 0 > gpurun_out/r2_bs1_traffic.log 2>&1
 tail -3 gpurun_out/r2_ncu_bs1_traffic.csv | cut -c1-200
 # full captures: prefill GEMM (tensor pipe), batched flash attention, small-batch mma kernel
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:gemm_i8_kernel -s 3 -c 1 -o gpurun_out/r2_gemm_i8 -f python tools/batched_prof.py pp512 2 1 > gpurun_out/r2_ncu_gemm.log 2>&1
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:gemv_mma_kernel -s 8 -c 1 -o gpurun_out/r2_gemv_mma -f python tools/batched_prof.py bs32 2 1 > gpurun_out/r2_ncu_mma.log 2>&1
 ls -la gpurun_out/*.ncu-rep
