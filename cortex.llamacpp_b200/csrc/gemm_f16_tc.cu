@@ -1,0 +1,224 @@
+// gemm_f16_tc.cu -- F16/BF16 weight matmul for prompt batches (more than 32 token columns) on the 5th-generation tensor cores:
+// tcgen05.mma cta_group::1 kind::f16 with f16 or bf16 operands (chosen by the instruction descriptor), f32 accumulators in TMEM.
+//   * x is rounded once per matmul to the weight's 16-bit type (the CPU's vec_dot_type, round-to-nearest-even) by a pack kernel that
+//     writes a dense [M][K] image into context scratch;
+//   * both operands come in through 2-D TMA tensor maps (SWIZZLE_128B, K-major, 64 k per stage): the weight tile of 128 rows straight
+//     from the GGUF rows, the activation tile of 128 tokens from the image.  The tensor maps' zero fill covers the N, M and K tails;
+//   * warp-specialised CTA of one 128 x 128 output tile: warp 0 issues the TMA loads into a ring of operand stages (full / empty
+//     mbarriers), warp 1 allocates TMEM and issues 4 MMAs of K = 16 per stage from one elected lane, warps 2..5 drain the accumulator
+//     (tcgen05.ld) and store f32;
+//   * when the tile grid leaves most SMs idle, K is split into slices whose partials a second kernel adds in slice order
+//     (deterministic).
+// Products of two 16-bit floats are exact in f32: the result differs from the CPU only in the order of the f32 additions.
+// Roofline: tensor pipe for prompt batches; algorithmic work 2 N K M flops, bytes 2 N K + 4 M K + 4 M N.
+#include "float_mm.h"
+#include "tc05.cuh"
+#include <cuda_bf16.h>
+#include <algorithm>
+
+namespace {
+
+constexpr int FT_M = 128, FT_N = 128, FT_K = 64;                 // weight rows, token columns, k per stage
+constexpr uint32_t FT_TILE = FT_M * FT_K * 2;                     // 16 KB per operand tile
+constexpr int FT_THREADS = 6 * 32;
+constexpr int FT_MAX_STAGES = 8;
+
+struct FtParams {
+    int N, M, K;
+    float *dst; size_t dst_stride;
+    float *part;                        // [ksplit][M][N] when gridDim.z > 1
+    int st_per_split, nst, nstages;     // k stages per slice, in all
+};
+
+struct FtBars { uint64_t full[FT_MAX_STAGES], empty[FT_MAX_STAGES], acc_full; uint32_t tmem_base; };
+
+template <bool BF>
+__global__ void __launch_bounds__(FT_THREADS, 1) b200_gemm_f16_tc_kernel(const __grid_constant__ CUtensorMap tmw, const __grid_constant__ CUtensorMap tmx,
+                                                                         const FtParams p) {
+    extern __shared__ uint8_t ft_smem_raw[];
+    uint8_t *smem = ft_smem_raw + ((1024u - (smem_u32(ft_smem_raw) & 1023u)) & 1023u);      // SWIZZLE_128B tiles: 1024-byte aligned
+    const int ns = p.nstages;
+    FtBars *S = (FtBars *)(smem + (size_t)ns * 2 * FT_TILE);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int row0 = blockIdx.x * FT_M, tok0 = blockIdx.y * FT_N;
+    const int st0 = blockIdx.z * p.st_per_split, nst = min(p.st_per_split, p.nst - st0);
+    if (threadIdx.x == 0) {
+        for (int i = 0; i < ns; i++) { mbar_init(&S->full[i], 1); mbar_init(&S->empty[i], 1); }
+        mbar_init(&S->acc_full, 1);
+        mbar_fence_init();
+    }
+    if (warp == 1) tmem_alloc(&S->tmem_base, FT_N);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = S->tmem_base;
+
+    if (warp == 0) {
+        // ------------------------------------------------------------ TMA producer: weight tile + activation tile per stage
+        for (int i = 0; i < nst; i++) {
+            const int st = i % ns, use = i / ns;
+            if (use > 0) mbar_wait_bounded(&S->empty[st], (use - 1) & 1);
+            if (elect_one_sync()) {
+                uint8_t *a = smem + (size_t)st * 2 * FT_TILE;
+                mbar_arrive_expect_tx(&S->full[st], 2 * FT_TILE);
+                tma_load_2d(a, &tmw, (st0 + i) * FT_K, row0, &S->full[st]);
+                tma_load_2d(a + FT_TILE, &tmx, (st0 + i) * FT_K, tok0, &S->full[st]);
+            }
+            __syncwarp();
+        }
+    } else if (warp == 1) {
+        // ------------------------------------------------------------ MMA issuer (warp-uniform loop, one elected lane issues)
+        constexpr uint32_t idesc = idesc_f16(BF, FT_M, FT_N);
+        const uint32_t base = smem_u32(smem);
+        for (int i = 0; i < nst; i++) {
+            const int st = i % ns, use = i / ns;
+            mbar_wait_bounded(&S->full[st], use & 1);
+            tc_fence_after();
+            if (elect_one_sync()) {
+                const uint32_t a = base + (uint32_t)st * 2 * FT_TILE, b = a + FT_TILE;
+#pragma unroll
+                for (int k = 0; k < FT_K / 16; k++)
+                    mma_f16(tmem, make_desc_sw128(a + 32 * k), make_desc_sw128(b + 32 * k), idesc, (i | k) ? 1u : 0u);
+                tc_commit(&S->empty[st]);                      // the stage is free once these MMAs have read it
+                if (i == nst - 1) tc_commit(&S->acc_full);     // the accumulator is complete
+            }
+            __syncwarp();
+        }
+    } else {
+        // ------------------------------------------------------------ drain: TMEM lane = weight row, column = token
+        const int q = warp & 3, row = row0 + q * 32 + lane;
+        mbar_wait_bounded(&S->acc_full, 0);
+        tc_fence_after();
+        float *const dstv = gridDim.z > 1 ? p.part + (size_t)blockIdx.z * p.M * p.N : p.dst;
+        const size_t stride = gridDim.z > 1 ? (size_t)p.N : p.dst_stride;
+#pragma unroll 1
+        for (int c0 = 0; c0 < FT_N; c0 += 32) {
+            uint32_t v[32];
+            tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);
+            tmem_ld_wait();
+            if (row < p.N)
+#pragma unroll
+                for (int j = 0; j < 32; j++) {
+                    const int tok = tok0 + c0 + j;
+                    if (tok < p.M) dstv[(size_t)tok * stride + row] = __uint_as_float(v[j]);
+                }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) tmem_dealloc(tmem, FT_N);
+}
+
+// x f32 [M] columns (stride x_stride floats) -> [M][K] image of 16-bit values, 8 elements per thread
+template <bool BF>
+__global__ void __launch_bounds__(256) b200_gemm_f16_pack_kernel(const float *__restrict__ x, size_t x_stride, int K, int M, uint16_t *__restrict__ img) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, k8 = K / 8;
+    if (i >= (int64_t)M * k8) return;
+    const int64_t m = i / k8, k = (i % k8) * 8;
+    const float4 a = *(const float4 *)(x + m * x_stride + k), b = *(const float4 *)(x + m * x_stride + k + 4);
+    uint32_t o[4];
+    if (BF) {
+        __nv_bfloat162 h[4] = {__floats2bfloat162_rn(a.x, a.y), __floats2bfloat162_rn(a.z, a.w), __floats2bfloat162_rn(b.x, b.y), __floats2bfloat162_rn(b.z, b.w)};
+        for (int j = 0; j < 4; j++) o[j] = *(uint32_t *)&h[j];
+    } else {
+        __half2 h[4] = {__floats2half2_rn(a.x, a.y), __floats2half2_rn(a.z, a.w), __floats2half2_rn(b.x, b.y), __floats2half2_rn(b.z, b.w)};
+        for (int j = 0; j < 4; j++) o[j] = *(uint32_t *)&h[j];
+    }
+    *(uint4 *)(img + m * (int64_t)K + k) = make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// dst[tok][n] = sum over the K slices in slice order (deterministic)
+__global__ void __launch_bounds__(256) b200_gemm_f16_reduce_kernel(const float *__restrict__ part, int ksplit, int N, int M, float *__restrict__ dst, size_t dst_stride) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)M * N) return;
+    float a = part[i];
+    for (int z = 1; z < ksplit; z++) a += part[(size_t)z * M * N + i];
+    dst[(i / N) * dst_stride + i % N] = a;
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
+                                  const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+template <bool BF>
+int launch_ft(b200_ctx *ctx, const CUtensorMap &tw, const CUtensorMap &tx, const FtParams &p, dim3 grid, size_t smem) {
+    auto kern = b200_gemm_f16_tc_kernel<BF>;
+    static bool attr_set[16] = {false};
+    if (!attr_set[ctx->device & 15]) {
+        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin));
+        attr_set[ctx->device & 15] = true;
+    }
+    kern<<<grid, FT_THREADS, smem, ctx->stream>>>(tw, tx, p);
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}
+
+}  // namespace
+
+int make_tmap_16bit(CUtensorMap *map, int type, const void *base, int64_t inner, int64_t outer, uint32_t box_inner, uint32_t box_outer) {
+    static EncodeTiledFn encode = nullptr;
+    if (!encode) {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !fn) {
+            cudaGetLastError();
+            b200_set_error("cuTensorMapEncodeTiled: driver entry point not found");
+            return B200_ERR_FAILED;
+        }
+        encode = (EncodeTiledFn)fn;
+    }
+    const cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)outer}, strides[1] = {(cuuint64_t)inner * 2};
+    const cuuint32_t box[2] = {box_inner, box_outer}, estr[2] = {1, 1};
+    const CUresult r = encode(map, type == B200_TYPE_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(base), dims, strides,
+                              box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { b200_set_error("cuTensorMapEncodeTiled failed (%d): %lld x %lld", (int)r, (long long)inner, (long long)outer); return B200_ERR_FAILED; }
+    return B200_OK;
+}
+
+int gemm_f16_tc_run(b200_ctx *ctx, int type, const uint16_t *W, int64_t N, int64_t K, const float *x, size_t x_stride_bytes, int64_t M, float *dst,
+                    size_t dst_stride) {
+    if ((type != B200_TYPE_F16 && type != B200_TYPE_BF16) || M < 1 || N < 1 || K % 8 || ((uintptr_t)W & 15) || ((uintptr_t)x & 15) || (x_stride_bytes & 15) ||
+        N > INT32_MAX || K > INT32_MAX || M > INT32_MAX) {
+        b200_set_error("gemm_f16_tc: unsupported shape");
+        return B200_ERR_UNSUPPORTED;
+    }
+    const bool bf = type == B200_TYPE_BF16;
+    uint16_t *img = (uint16_t *)ctx->get_scratch(SCRATCH_ACT, (size_t)M * K * 2);
+    if (!img) return B200_ERR_ALLOC;
+    {
+        const int64_t n = M * (K / 8);
+        if (bf) b200_gemm_f16_pack_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(x, x_stride_bytes / 4, (int)K, (int)M, img);
+        else    b200_gemm_f16_pack_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(x, x_stride_bytes / 4, (int)K, (int)M, img);
+        ctx->launches++;
+        CUDA_TRY(cudaGetLastError());
+    }
+    CUtensorMap tw, tx;
+    int rc = make_tmap_16bit(&tw, type, W, K, N, FT_K, FT_M);
+    if (!rc) rc = make_tmap_16bit(&tx, type, img, K, M, FT_K, FT_N);
+    if (rc) return rc;
+    FtParams p = {};
+    p.N = (int)N; p.M = (int)M; p.K = (int)K; p.dst = dst; p.dst_stride = dst_stride;
+    p.nst = (int)((K + FT_K - 1) / FT_K);
+    const size_t fixed = 1024 + sizeof(FtBars);
+    p.nstages = (int)std::min<size_t>(FT_MAX_STAGES, (ctx->smem_optin - fixed) / (2 * FT_TILE));
+    // split K when the tile grid covers less than half of the SMs: slices of >= 8 stages (512 k), partials reduced in slice order
+    const int64_t ctas = ((N + FT_M - 1) / FT_M) * ((M + FT_N - 1) / FT_N);
+    int ksplit = 1;
+    while (ksplit < 8 && ctas * ksplit * 2 <= ctx->sm_count && p.nst / (ksplit * 2) >= 8) ksplit *= 2;
+    p.st_per_split = (p.nst + ksplit - 1) / ksplit;
+    ksplit = (p.nst + p.st_per_split - 1) / p.st_per_split;
+    if (ksplit > 1) {
+        p.part = (float *)ctx->get_scratch(SCRATCH_MISC, (size_t)ksplit * M * N * 4);
+        if (!p.part) return B200_ERR_ALLOC;
+    }
+    const dim3 grid((unsigned)((N + FT_M - 1) / FT_M), (unsigned)((M + FT_N - 1) / FT_N), (unsigned)ksplit);
+    const size_t smem = fixed + (size_t)p.nstages * 2 * FT_TILE;
+    rc = bf ? launch_ft<true>(ctx, tw, tx, p, grid, smem) : launch_ft<false>(ctx, tw, tx, p, grid, smem);
+    if (rc || ksplit == 1) return rc;
+    const int64_t total = M * N;
+    b200_gemm_f16_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx->stream>>>(p.part, ksplit, (int)N, (int)M, dst, dst_stride);
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}

@@ -595,9 +595,10 @@ extern "C" int b200_graph_compute(b200_ctx *ctx, const b200_op *ops, int n_ops) 
         bool decode_like = false;
         for (const ExecNode &x : list) {
             decode_like |= x.kind == EX_GEMV;
-            // a continuous-batching step (<= 32 token columns) repeats like a decode step
+            // a continuous-batching step (<= 32 token columns) repeats like a decode step; F16/BF16 weights (unfused) included
+            const int wt = x.op.src[0].type;
             decode_like |= x.kind == EX_OP && x.op.op == B200_OP_MUL_MAT && x.op.src[1].ne[1] <= 32 && (x.op.src[0].flags & B200_TENSOR_FLAG_WEIGHT) &&
-                           b200_type_is_quant(x.op.src[0].type);
+                           (b200_type_is_quant(wt) || wt == B200_TYPE_F16 || wt == B200_TYPE_BF16);
         }
         if (!decode_like && ctx->opt_fusion >= 2) return run_list(ctx, list);
     }

@@ -9,7 +9,10 @@
 //   quantised W, M > 32      : K-quants: tcgen05 kind::f16 GEMM (gemm_tc.cu); other formats: prompt-batch GEMM on mma.sync (gemm_mma.cu);
 //                              shapes neither takes (N % 128, K % 256): GEMV in column chunks
 //   row-split W (B200_TENSOR_FLAG_SPLIT): every shard's GPU at once (op_mul_mat_split)
-//   F32/F16/BF16 W           : warp-per-row float kernel below (MoE router, small test shapes)
+//   F16/BF16 W, rows contiguous and 16-byte aligned, K % 8 == 0 (float_mm_ok):
+//                       M <= 32: weight-streaming mma.sync kernel, x rounded to the weight type in its prologue (gemv_f16.cu)
+//                       M > 32 : rounded x image + tcgen05 kind::f16 GEMM over TMA tiles (gemm_f16_tc.cu)
+//   F32 W, other F16/BF16 layouts (strided or permuted views, odd K, unaligned operands): warp-per-row float kernel below
 //   cpu_exact mode           : exact.cu (the reference AVX2 build's summation order)
 // MUL_MAT_ID: device-side expert routing -- no host sync on `ids` (the reference copies ids to the host and loops experts there):
 // one GEMV per (token, slot) for decode-sized batches, pairs grouped by expert on the device + grouped gemv_mma for batches.
@@ -17,6 +20,7 @@
 #include <algorithm>
 #include <cuda_bf16.h>
 #include "gemm_tc.h"
+#include "float_mm.h"
 
 int gemv_max_cols(const b200_ctx *ctx, int type, size_t rb, int64_t K);
 int launch_gemv_f32(b200_ctx *ctx, int type, const uint8_t *W, size_t row_bytes, int64_t N, int64_t K, const float *x, size_t x_stride_bytes,
@@ -135,6 +139,34 @@ bool quant_mul_mat_shape_ok(const b200_tensor &w, const b200_tensor &x, const b2
     return true;
 }
 
+// F16/BF16 weights that the tensor-core kernels take: contiguous 16-byte aligned rows (TMA tiles), K % 8 == 0, f32 x with 16-byte
+// aligned columns (float4 loads), f32 dst columns
+bool float_mm_ok(const b200_ctx *ctx, const b200_tensor &w, const b200_tensor &x, const b200_tensor &d) {
+    if (ctx->opt_cpu_exact || (w.type != B200_TYPE_F16 && w.type != B200_TYPE_BF16)) return false;
+    const int64_t K = w.ne[0];
+    if (K % 8 || w.nb[0] != 2 || w.nb[1] != (uint64_t)K * 2 || (((uintptr_t)w.data | w.nb[2] | w.nb[3]) & 15)) return false;
+    if (x.type != B200_TYPE_F32 || x.ne[0] != K || x.nb[0] != 4 || (((uintptr_t)x.data | x.nb[1] | x.nb[2] | x.nb[3]) & 15)) return false;
+    if (d.type != B200_TYPE_F32 || d.nb[0] != 4 || ((d.nb[1] | d.nb[2] | d.nb[3]) & 3)) return false;
+    return w.ne[2] > 0 && w.ne[3] > 0 && x.ne[2] % w.ne[2] == 0 && x.ne[3] % w.ne[3] == 0;
+}
+
+int mul_mat_f16_tc(b200_ctx *ctx, const b200_tensor &w, const b200_tensor &x, const b200_tensor &d) {
+    const int64_t K = w.ne[0], N = w.ne[1], M = x.ne[1];
+    if (tensor_nelements(d) == 0) return B200_OK;
+    const bool w_const = (w.flags & B200_TENSOR_FLAG_WEIGHT) != 0;
+    for (int64_t i3 = 0; i3 < x.ne[3]; i3++)
+        for (int64_t i2 = 0; i2 < x.ne[2]; i2++) {
+            const int64_t w2 = i2 / (x.ne[2] / w.ne[2]), w3 = i3 / (x.ne[3] / w.ne[3]);
+            const uint16_t *wp = (const uint16_t *)((const char *)w.data + w2 * w.nb[2] + w3 * w.nb[3]);
+            const float *xp = (const float *)((const char *)x.data + i2 * x.nb[2] + i3 * x.nb[3]);
+            float *dp = (float *)((char *)d.data + i2 * d.nb[2] + i3 * d.nb[3]);
+            const int rc = M <= F16MM_STREAM_MAX_M ? gemv_f16_run(ctx, w.type, wp, N, K, xp, x.nb[1], (int)M, dp, d.nb[1] / 4, w_const)
+                                                   : gemm_f16_tc_run(ctx, w.type, wp, N, K, xp, x.nb[1], M, dp, d.nb[1] / 4);
+            if (rc) return rc;
+        }
+    return B200_OK;
+}
+
 }  // namespace
 
 // row-split weight: the shard of every device is a dense GGUF matrix of its row range
@@ -214,7 +246,7 @@ static int op_mul_mat_split(b200_ctx *ctx, const b200_op *op) {
 int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
     const b200_tensor &w = op->src[0], &x = op->src[1], &d = op->dst;
     if (w.flags & B200_TENSOR_FLAG_SPLIT) return op_mul_mat_split(ctx, op);
-    if (!b200_type_is_quant(w.type)) return mul_mat_float(ctx, w, x, d);
+    if (!b200_type_is_quant(w.type)) return float_mm_ok(ctx, w, x, d) ? mul_mat_f16_tc(ctx, w, x, d) : mul_mat_float(ctx, w, x, d);
     if (!quant_mul_mat_shape_ok(w, x, d)) { b200_set_error("mul_mat: unsupported layout"); return B200_ERR_UNSUPPORTED; }
     const int64_t K = w.ne[0], N = w.ne[1], M = x.ne[1];
     const int q8k = b200_act_mode_q8k(w.type);

@@ -19,8 +19,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tools"))
 from make_gguf import MODELS, tensor_type  # noqa: E402
 
-F32, F16, Q4_0, Q8_0, Q4_K, Q5_K, Q6_K, I32 = 0, 1, 2, 8, 12, 13, 14, 26
-BLOCK = {F32: (1, 4), F16: (1, 2), I32: (1, 4), Q4_0: (32, 18), Q8_0: (32, 34), Q4_K: (256, 144), Q5_K: (256, 176), Q6_K: (256, 210)}
+F32, F16, Q4_0, Q8_0, Q4_K, Q5_K, Q6_K, I32, BF16 = 0, 1, 2, 8, 12, 13, 14, 26, 30
+BLOCK = {F32: (1, 4), F16: (1, 2), BF16: (1, 2), I32: (1, 4), Q4_0: (32, 18), Q8_0: (32, 34), Q4_K: (256, 144), Q5_K: (256, 176), Q6_K: (256, 210)}
 KV_TYPES = {"f16": F16, "q8_0": Q8_0, "q4_0": Q4_0}
 
 
@@ -28,6 +28,17 @@ def row_size(t, k):
     be, bb = BLOCK[t]
     assert k % be == 0, (t, k)
     return k // be * bb
+
+
+def device_rand_16bit(torch, t, nrows, K, amp, gen, device):
+    """uniform(-amp, amp) weights of F16 / BF16 type ``t`` created in HBM, as raw bytes"""
+    dt = torch.float16 if t == F16 else torch.bfloat16
+    out = torch.empty(nrows * K, dtype=dt, device=device)
+    step = 1 << 26
+    for i0 in range(0, nrows * K, step):
+        n = min(step, nrows * K - i0)
+        out[i0:i0 + n] = ((torch.rand(n, device=device, generator=gen) * 2 - 1) * amp).to(dt)
+    return out.view(torch.uint8)
 
 
 def device_rand_blocks(torch, t, nrows, K, amp, gen, device):
@@ -132,6 +143,8 @@ class LlamaGraph:
             amp = gain * math.sqrt(3.0 / K)
             if t == F32:
                 buf = ((torch.rand(N * K, device=self.dev, generator=gen) * 2 - 1) * amp).view(torch.uint8)
+            elif t in (F16, BF16):
+                buf = device_rand_16bit(torch, t, N, K, amp, gen, self.dev)
             else:
                 buf = device_rand_blocks(torch, t, N, K, amp, gen, self.dev)
             if tp_world > 1 and split == "rows":
@@ -149,7 +162,10 @@ class LlamaGraph:
         def experts(name, K, N, il):
             """n_expert matrices [K, N] back to back (ggml layout [K, N, n_expert], llama-model.cpp ffn_*_exps)"""
             t = tensor_type(name, ftype, il, L, n_expert, Hf // Hkvf)
-            buf = device_rand_blocks(torch, t, N * n_expert, K, math.sqrt(3.0 / K), gen, self.dev)
+            if t in (F16, BF16):
+                buf = device_rand_16bit(torch, t, N * n_expert, K, math.sqrt(3.0 / K), gen, self.dev)
+            else:
+                buf = device_rand_blocks(torch, t, N * n_expert, K, math.sqrt(3.0 / K), gen, self.dev)
             self.keep.append(buf)
             nbytes = n_expert * N * row_size(t, K)
             self.weight_bytes += nbytes

@@ -16,9 +16,9 @@ import sys
 
 import numpy as np
 
-F32, F16, Q4_0, Q8_0, Q4_K, Q5_K, Q6_K = 0, 1, 2, 8, 12, 13, 14
-BLOCK = {F32: (1, 4), F16: (1, 2), Q4_0: (32, 18), Q8_0: (32, 34), Q4_K: (256, 144), Q5_K: (256, 176), Q6_K: (256, 210)}
-FTYPE_ID = {"f32": 0, "q4_0": 2, "q8_0": 7, "q4_k_m": 15, "q5_k_m": 17}
+F32, F16, Q4_0, Q8_0, Q4_K, Q5_K, Q6_K, BF16 = 0, 1, 2, 8, 12, 13, 14, 30
+BLOCK = {F32: (1, 4), F16: (1, 2), BF16: (1, 2), Q4_0: (32, 18), Q8_0: (32, 34), Q4_K: (256, 144), Q5_K: (256, 176), Q6_K: (256, 210)}
+FTYPE_ID = {"f32": 0, "f16": 1, "bf16": 32, "q4_0": 2, "q8_0": 7, "q4_k_m": 15, "q5_k_m": 17}
 
 MODELS = {
     #               L   E     H   Hkv D    FF     V       rope_base  n_expert n_used
@@ -44,6 +44,8 @@ def tensor_type(name, ftype, i_layer, n_layer, n_expert, n_gqa):
         return F32
     if ftype == "f32":
         return F32
+    if ftype in ("f16", "bf16"):              # MOSTLY_F16 / MOSTLY_BF16: every matmul weight and token_embd
+        return F16 if ftype == "f16" else BF16
     base = {"q4_0": Q4_0, "q8_0": Q8_0, "q4_k_m": Q4_K, "q5_k_m": Q5_K}[ftype]
     if name == "output.weight":
         return Q8_0 if ftype == "q8_0" else Q6_K
@@ -62,6 +64,14 @@ def tensor_type(name, ftype, i_layer, n_layer, n_expert, n_gqa):
         if "attn_output.weight" in name and n_expert == 8 and ftype == "q4_k_m":
             return Q5_K
     return base
+
+
+def to_16bit(t, x):
+    """f32 array -> F16 or BF16 (round-to-nearest-even, as ggml_compute_fp32_to_bf16 for finite values) as uint16"""
+    if t == F16:
+        return x.astype(np.float16).view(np.uint16)
+    u = x.astype(np.float32).view(np.uint32).astype(np.uint64)
+    return ((u + 0x7FFF + ((u >> 16) & 1)) >> 16).astype(np.uint16)
 
 
 def rand_blocks(t, nrows, K, rng, amp):
@@ -209,6 +219,8 @@ def main():
                 nr = min(step, rows_total - r0)
                 if t == F32:
                     yield (rng.uniform(-amp, amp, nr * K)).astype(np.float32)
+                elif t in (F16, BF16):
+                    yield to_16bit(t, rng.uniform(-amp, amp, nr * K).astype(np.float32))
                 else:
                     yield rand_blocks(t, nr, K, rng, amp)
         w.tensor(name, ne, t, gen)
