@@ -15,7 +15,12 @@
 //   F32 W, other F16/BF16 layouts (strided or permuted views, odd K, unaligned operands): warp-per-row float kernel below
 //   cpu_exact mode           : exact.cu (the reference AVX2 build's summation order)
 // MUL_MAT_ID: device-side expert routing -- no host sync on `ids` (the reference copies ids to the host and loops experts there):
-// one GEMV per (token, slot) for decode-sized batches, pairs grouped by expert on the device + grouped gemv_mma for batches.
+//   quantised experts: one GEMV per (token, slot) for decode-sized batches, pairs grouped by expert on the device + grouped gemv_mma for
+//                      batches, grouped tile GEMMs for prompt batches;
+//   F16/BF16 experts, rows contiguous and 16-byte aligned, K % 8 == 0, dense x (float_mm_id_ok): pairs grouped by expert on the device
+//                      at every batch size, then < 32 pairs per expert on average: grouped weight-streaming kernel (gemv_f16.cu);
+//                      more: grouped tcgen05 GEMM over a pair-sorted rounded image (gemm_f16_tc.cu);
+//   F32 experts, other F16/BF16 layouts, cpu_exact mode: warp-per-(row, pair) float kernel reading the expert from ids on the device.
 #include "common.cuh"
 #include <algorithm>
 #include <cuda_bf16.h>
@@ -106,6 +111,44 @@ int mul_mat_float(b200_ctx *ctx, const b200_tensor &w, const b200_tensor &x, con
         case B200_TYPE_F32:  b200_mul_mat_float_kernel<float><<<grid, 128, 0, ctx->stream>>>(w, x, d); break;
         case B200_TYPE_F16:  b200_mul_mat_float_kernel<__half><<<grid, 128, 0, ctx->stream>>>(w, x, d); break;
         case B200_TYPE_BF16: b200_mul_mat_float_kernel<__nv_bfloat16><<<grid, 128, 0, ctx->stream>>>(w, x, d); break;
+        default: return B200_ERR_UNSUPPORTED;
+    }
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}
+
+// MUL_MAT_ID with float experts, the arithmetic of b200_mul_mat_float_kernel: one warp per (row n, slot, token); the expert index is read
+// from ids on the device (an index outside [0, E) leaves its dst column untouched, as the grouped paths do)
+template <typename WT>
+__global__ void __launch_bounds__(128) b200_mul_mat_id_float_kernel(b200_tensor as, b200_tensor b, b200_tensor ids, b200_tensor d) {
+    const int lane = threadIdx.x & 31;
+    const int64_t gw = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int64_t N = d.ne[0], n_used = d.ne[1];
+    if (gw >= N * n_used * d.ne[2]) return;
+    const int64_t n = gw % N, s = (gw / N) % n_used, t = gw / (N * n_used);
+    const int e = *(const int32_t *)((const char *)ids.data + s * ids.nb[0] + t * ids.nb[1]);
+    if (e < 0 || e >= as.ne[2]) return;
+    const char *wp = (const char *)as.data + n * as.nb[1] + (int64_t)e * as.nb[2];
+    const char *xp = (const char *)b.data + (s % b.ne[1]) * b.nb[1] + t * b.nb[2];
+    float acc = 0.0f;
+    for (int64_t k = lane; k < as.ne[0]; k += 32) {
+        const float wv = w_to_float<WT>(*(const WT *)(wp + k * as.nb[0]));
+        const float xv = x_round<WT>(*(const float *)(xp + k * b.nb[0]));
+        acc = fmaf(wv, xv, acc);
+    }
+    acc = warp_reduce_sum(acc);
+    if (lane == 0) *(float *)((char *)d.data + n * d.nb[0] + s * d.nb[1] + t * d.nb[2]) = acc;
+}
+
+int mul_mat_id_float(b200_ctx *ctx, const b200_tensor &as, const b200_tensor &b, const b200_tensor &ids, const b200_tensor &d) {
+    const int64_t total = d.ne[0] * d.ne[1] * d.ne[2];
+    if (total == 0) return B200_OK;
+    const unsigned grid = (unsigned)((total + 3) / 4);
+    switch (as.type) {
+        case B200_TYPE_F32:  b200_mul_mat_id_float_kernel<float><<<grid, 128, 0, ctx->stream>>>(as, b, ids, d); break;
+        case B200_TYPE_F16:  b200_mul_mat_id_float_kernel<__half><<<grid, 128, 0, ctx->stream>>>(as, b, ids, d); break;
+        case B200_TYPE_BF16: b200_mul_mat_id_float_kernel<__nv_bfloat16><<<grid, 128, 0, ctx->stream>>>(as, b, ids, d); break;
         default: return B200_ERR_UNSUPPORTED;
     }
     ctx->launches++;
@@ -363,7 +406,14 @@ int op_mul_mat(b200_ctx *ctx, const b200_op *op) {
 // ---------------------------------------------------------------------------------------------------
 bool supports_mul_mat_id(const b200_op *op) {
     const b200_tensor &as = op->src[0], &b = op->src[1], &ids = op->src[2], &d = op->dst;
-    if (!b200_type_is_quant(as.type) || b.type != B200_TYPE_F32 || d.type != B200_TYPE_F32 || ids.type != B200_TYPE_I32) return false;
+    if (b.type != B200_TYPE_F32 || d.type != B200_TYPE_F32 || ids.type != B200_TYPE_I32) return false;
+    const bool fl = as.type == B200_TYPE_F32 || as.type == B200_TYPE_F16 || as.type == B200_TYPE_BF16;
+    if (fl) {                  // any strides: what the tensor-core paths do not take, the float kernel does
+        if (as.ne[3] != 1 || b.ne[3] != 1 || d.ne[3] != 1 || b.ne[0] != as.ne[0]) return false;
+        if (d.ne[0] != as.ne[1] || d.ne[1] != ids.ne[0] || d.ne[2] != ids.ne[1] || b.ne[2] != ids.ne[1]) return false;
+        return b.ne[1] == 1 || b.ne[1] == ids.ne[0];
+    }
+    if (!b200_type_is_quant(as.type)) return false;
     const int64_t K = as.ne[0];
     if (K % b200_type_block_elems(as.type) != 0 || K % 32 != 0 || b.ne[0] != K) return false;
     if (as.nb[0] != (uint64_t)b200_type_block_bytes(as.type) || as.nb[1] != b200_row_bytes(as.type, K)) return false;
@@ -409,8 +459,44 @@ __global__ void __launch_bounds__(1024) b200_moe_group_kernel(const char *ids, u
     }
 }
 
+// F16/BF16 experts that the grouped tensor-core paths take: contiguous 16-byte aligned expert rows (3-D TMA map), K % 8 == 0, x columns
+// of the pairs 16-byte aligned and dense across tokens (float4 gathers), f32 dst; the routing tables' limits (one grouping CTA)
+static bool float_mm_id_ok(const b200_ctx *ctx, const b200_tensor &as, const b200_tensor &b, const b200_tensor &ids, const b200_tensor &d) {
+    if (ctx->opt_cpu_exact || (as.type != B200_TYPE_F16 && as.type != B200_TYPE_BF16)) return false;
+    const int64_t K = as.ne[0], npairs = ids.ne[0] * ids.ne[1];
+    if (K % 8 || K > INT32_MAX || as.ne[1] > INT32_MAX || as.nb[0] != 2 || as.nb[1] != (uint64_t)K * 2 || (((uintptr_t)as.data | as.nb[2]) & 15)) return false;
+    const bool b_dense = b.ne[1] == 1 || b.nb[2] == b.ne[1] * b.nb[1];
+    if (!b_dense || b.nb[0] != 4 || (((uintptr_t)b.data | b.nb[1] | b.nb[2]) & 15)) return false;
+    if (d.nb[0] != 4 || ((d.nb[1] | d.nb[2]) & 3)) return false;
+    return as.ne[2] >= 1 && as.ne[2] <= 1024 && npairs >= 1 && npairs <= (1 << 20);
+}
+
+// MUL_MAT_ID with F32 / F16 / BF16 experts
+static int op_mul_mat_id_float(b200_ctx *ctx, const b200_tensor &as, const b200_tensor &b, const b200_tensor &ids, const b200_tensor &d) {
+    if (!float_mm_id_ok(ctx, as, b, ids, d)) return mul_mat_id_float(ctx, as, b, ids, d);
+    const int64_t K = as.ne[0], N = as.ne[1], npairs = ids.ne[0] * ids.ne[1], E = as.ne[2];
+    int32_t *tab = (int32_t *)ctx->get_scratch(SCRATCH_MOE, (size_t)(E + 1 + npairs) * 4);
+    if (!tab) return B200_ERR_ALLOC;
+    b200_moe_group_kernel<<<1, 1024, (size_t)2 * E * sizeof(int), ctx->stream>>>((const char *)ids.data, ids.nb[0], ids.nb[1], (int)ids.ne[0], (int)ids.ne[1], (int)E, tab, tab + E + 1, 0);
+    ctx->launches++;
+    CUDA_TRY(cudaGetLastError());
+    MmGroupDesc g = {};
+    g.off = tab; g.pairs = tab + E + 1; g.E = (int)E; g.n_used = (int)ids.ne[0]; g.b_ne1 = (int)b.ne[1];
+    g.expert_stride = as.nb[2]; g.d_nb1 = d.nb[1] / 4; g.d_nb2 = d.nb[2] / 4;
+    const size_t x_stride = b.ne[1] == 1 ? b.nb[2] : b.nb[1];
+    // prompt batches (>= 32 pairs per expert on average): token tiles of 128 pairs per expert through the tcgen05 GEMM, as for quantised
+    // experts (profiles/moe_float_weights.md)
+    if (npairs >= 32 * E) {
+        g.max_chunks = (int)std::min<int64_t>(npairs, npairs / 128 + E);
+        return gemm_f16_tc_run_grouped(ctx, as.type, (const uint16_t *)as.data, N, K, (const float *)b.data, x_stride, g, npairs, (float *)d.data);
+    }
+    g.max_chunks = (int)std::min<int64_t>(npairs, npairs / 32 + E);
+    return gemv_f16_run_grouped(ctx, as.type, (const uint16_t *)as.data, N, K, (const float *)b.data, x_stride, g, npairs, (float *)d.data);
+}
+
 int op_mul_mat_id(b200_ctx *ctx, const b200_op *op) {
     const b200_tensor &as = op->src[0], &b = op->src[1], &ids = op->src[2], &d = op->dst;
+    if (!b200_type_is_quant(as.type)) return op_mul_mat_id_float(ctx, as, b, ids, d);
     const int64_t K = as.ne[0], N = as.ne[1], n_used = ids.ne[0], n_tok = ids.ne[1];
     const size_t rb = b200_row_bytes(as.type, K);
     // batches: group the (token, slot) pairs by expert on the device and stream every expert's matrix once per 32 pairs (the reference

@@ -1,6 +1,6 @@
 // tc05.cuh -- tcgen05 / TMEM / UMMA shared-memory descriptor primitives (inline PTX) shared by the tensor-core kernels
 // (gemm_tc.cu: kind::f16 GEMM with exact-integer f16 operands, fattn_tc.cu: flash attention, gemm_f16_tc.cu: F16/BF16 weight GEMM)
-// and the 2-D TMA tile load the F16/BF16 weight kernels stream through (gemm_f16_tc.cu, gemv_f16.cu).
+// and the 2-D / 3-D TMA tile loads the F16/BF16 weight kernels stream through (gemm_f16_tc.cu, gemv_f16.cu).
 #pragma once
 #include "common.cuh"
 
@@ -109,5 +109,12 @@ __device__ __forceinline__ bool elect_one_sync() {
 __device__ __forceinline__ void tma_load_2d(void *smem_dst, const void *tmap, int c0, int c1, uint64_t *bar) {
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(smem_u32(smem_dst)),
                  "l"((uint64_t)(uintptr_t)tmap), "r"(c0), "r"(c1), "r"(smem_u32(bar))
+                 : "memory");
+}
+// 3-D TMA tile load: box at (c0 = inner, c1 = outer, c2 = depth), e.g. (k, row, expert) of a stack of expert matrices; with a box depth
+// of 1 the shared-memory image is that of the 2-D box, and the zero fill stops at each matrix's own last row
+__device__ __forceinline__ void tma_load_3d(void *smem_dst, const void *tmap, int c0, int c1, int c2, uint64_t *bar) {
+    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(smem_u32(smem_dst)),
+                 "l"((uint64_t)(uintptr_t)tmap), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar))
                  : "memory");
 }
