@@ -114,6 +114,13 @@ static bool overlaps(const b200_tensor &a, const b200_tensor &b) {
     tensor_range(a, al, ah); tensor_range(b, bl, bh);
     return al < bh && bl < ah;
 }
+// does tensor a span every byte of tensor t?  (a write of a dense a then replaces t's whole value; a mere overlap leaves some of it)
+static bool covers(const b200_tensor &a, const b200_tensor &t) {
+    if (!a.data || !t.data) return false;
+    uintptr_t al, ah, tl, th;
+    tensor_range(a, al, ah); tensor_range(t, tl, th);
+    return al <= tl && th <= ah;
+}
 // is the VALUE currently held by tensor t still needed by ops[from..n)?  (first touch of its bytes: a read => yes, a write => no)
 static bool live_after(const b200_op *ops, int n, int from, const b200_tensor &t) {
     for (int i = from; i < n; i++) {
@@ -232,7 +239,7 @@ static int match_attention(b200_ctx *ctx, const b200_op *ops, int n, int i, cons
     //  which we do write: not a use of the intermediate)
     for (const b200_tensor *t : dead) if (live_after(ops, n, fa_idx, *t)) {
         bool reused = false;
-        for (int x = 0; x < nextra; x++) reused |= overlaps(*t, extra[x]->dst);
+        for (int x = 0; x < nextra; x++) reused |= covers(extra[x]->dst, *t);
         if (!reused) MA_FAIL(16);
     }
     (void)ctx;
@@ -297,13 +304,13 @@ static int match_ffn(const b200_op *ops, int n, int i, const FuseScratch &fs, st
     if (tp) {
         if (add.src[0].data != down->dst.data || !is_vec_f32(down->dst, E) || up->src[0].ne[1] != FF || down->src[0].ne[0] != FF) return 0;
         const b200_tensor *dead[] = {&ops[i].dst, &B, &gate->dst, &silu->dst, &up->dst, &mul->dst};
-        for (const b200_tensor *t : dead) if (!overlaps(*t, down->dst) && live_after(ops, n, i + 7, *t)) return 0;
+        for (const b200_tensor *t : dead) if (!covers(down->dst, *t) && live_after(ops, n, i + 7, *t)) return 0;
     } else {
         resid = add.src[0].data == down->dst.data ? &add.src[1] : (add.src[1].data == down->dst.data ? &add.src[0] : nullptr);
         if (!resid) return 0;
         if (up->src[0].ne[1] != FF || down->src[0].ne[0] != FF || !is_vec_f32(*resid, E) || !is_vec_f32(add.dst, E) || resid->ne[1] != T || add.dst.ne[1] != T) return 0;
         const b200_tensor *dead[] = {&ops[i].dst, &B, &gate->dst, &silu->dst, &up->dst, &mul->dst, &down->dst};
-        for (const b200_tensor *t : dead) if (!overlaps(*t, add.dst) && live_after(ops, n, i + 8, *t)) return 0;
+        for (const b200_tensor *t : dead) if (!covers(add.dst, *t) && live_after(ops, n, i + 8, *t)) return 0;
     }
     ExecNode g;
     g.kind = EX_GEMV; g.nseg = 2; g.K = xin->ne[0]; g.ncols = (int)T; g.w_const = true;
@@ -332,7 +339,7 @@ static int match_mm_add(const b200_op *ops, int n, int i, std::vector<ExecNode> 
     const int64_t N = mm.src[0].ne[1], T = mm.dst.ne[1];
     if (!resid || !is_vec_f32(*resid, N) || !is_vec_f32(add.dst, N) || resid->ne[1] != T || add.dst.ne[1] != T) return 0;
     if (overlaps(add.dst, mm.src[1])) return 0;
-    if (!overlaps(mm.dst, add.dst) && live_after(ops, n, i + 2, mm.dst)) return 0;
+    if (!covers(add.dst, mm.dst) && live_after(ops, n, i + 2, mm.dst)) return 0;
     ExecNode g;
     g.kind = EX_GEMV; g.nseg = 1; g.K = mm.src[0].ne[0]; g.ncols = (int)T; g.w_const = true;
     g.seg[0] = seg_of(mm, (float *)add.dst.data, (size_t)N, (const float *)resid->data);
