@@ -57,6 +57,10 @@ static int dispatch(b200_ctx *ctx, const b200_op *op) {
 extern "C" int b200_supports_op(int device, const b200_op *op) {
     (void)device;
     if (!op) return 0;
+    // a row-split tensor's `data` is the host-side b200_split: only op_mul_mat_split reads it, as the weight of a MUL_MAT
+    for (int i = 0; i < op->n_src && i < B200_MAX_SRC; i++)
+        if ((op->src[i].flags & B200_TENSOR_FLAG_SPLIT) && (op->op != B200_OP_MUL_MAT || i != 0)) return 0;
+    if (op->dst.flags & B200_TENSOR_FLAG_SPLIT) return 0;
     switch (op->op) {
         case B200_OP_NONE: return 1;
         case B200_OP_MUL_MAT: return supports_mul_mat(op) ? 1 : 0;

@@ -8,7 +8,7 @@
 //   quantised W, 5 <= M <= 32: quantise (quant.cu) + small-batch mma.sync kernel (gemv_mma.cu)
 //   quantised W, M > 32      : K-quants: tcgen05 kind::f16 GEMM (gemm_tc.cu); other formats: prompt-batch GEMM on mma.sync (gemm_mma.cu);
 //                              shapes neither takes (N % 128, K % 256): GEMV in column chunks
-//   row-split W (B200_TENSOR_FLAG_SPLIT): every shard's GPU at once (op_mul_mat_split)
+//   row-split W (B200_TENSOR_FLAG_SPLIT; quantised, F16, BF16): every shard's GPU at once (op_mul_mat_split)
 //   F16/BF16 W, rows contiguous and 16-byte aligned, K % 8 == 0 (float_mm_ok):
 //                       M <= 32: weight-streaming mma.sync kernel, x rounded to the weight type in its prologue (gemv_f16.cu)
 //                       M > 32 : rounded x image + tcgen05 kind::f16 GEMM over TMA tiles (gemm_f16_tc.cu)
@@ -216,9 +216,14 @@ int mul_mat_f16_tc(b200_ctx *ctx, const b200_tensor &w, const b200_tensor &x, co
 static bool split_ok(const b200_op *op) {
     const b200_tensor &w = op->src[0], &x = op->src[1], &d = op->dst;
     const b200_split *sp = (const b200_split *)w.data;
+    const bool f16 = w.type == B200_TYPE_F16 || w.type == B200_TYPE_BF16;
     // sp == NULL: llama.cpp probing whether a weight may live in the split buffer type (no shards allocated yet)
-    if ((sp && (sp->n_dev < 1 || sp->n_dev > B200_MAX_SPLIT)) || !b200_type_is_quant(w.type)) return false;
+    if ((sp && (sp->n_dev < 1 || sp->n_dev > B200_MAX_SPLIT)) || !(b200_type_is_quant(w.type) || f16)) return false;
     if (w.ne[2] != 1 || w.ne[3] != 1 || x.ne[2] != 1 || x.ne[3] != 1) return false;
+    // F16/BF16: dense shard rows; any f32 x and dst columns (layouts the tensor-core kernels refuse take the float kernel on every
+    // shard); dst rows 4 bytes apart, so that a shard's row range starts row_low * 4 bytes into dst
+    if (f16)
+        return w.nb[0] == 2 && w.nb[1] == (uint64_t)w.ne[0] * 2 && x.type == B200_TYPE_F32 && x.ne[0] == w.ne[0] && d.type == B200_TYPE_F32 && d.nb[0] == 4;
     b200_tensor w0 = w;                                   // shape checks against an aligned stand-in for the shards (cudaMalloc'd: 256-byte aligned)
     w0.data = (void *)(uintptr_t)0x1000; w0.flags &= ~B200_TENSOR_FLAG_SPLIT;
     return quant_mul_mat_shape_ok(w0, x, d);
@@ -236,8 +241,10 @@ bool supports_mul_mat(const b200_op *op) {
 
 // MUL_MAT over a row-split weight (replaces the split path of ggml_cuda_op_mul_mat, ggml-cuda.cu:1363-1671): fork on the main stream,
 // every device multiplies its shard into its row range of dst -- activations read from and results written to the MAIN device's memory
-// through NVLink peer access, no staging copies -- and the main stream joins.  Each dst element is produced by the same kernels as on
-// one GPU, so the result does not depend on the split.
+// through NVLink peer access, no staging copies -- and the main stream joins.  Quantised weights: each dst element is produced by the
+// same kernels as on one GPU, so the result does not depend on the split.  F16/BF16 weights: gemv_f16 and gemm_f16_tc choose their K
+// slices from the row count they are given, so a shard may sum K in other slices than the whole matrix would: the result equals the
+// one-GPU result up to f32 summation order, and is the same bits on every run of the same split.
 static int op_mul_mat_split(b200_ctx *ctx, const b200_op *op) {
     const b200_tensor &w = op->src[0];
     const b200_split *sp = (const b200_split *)w.data;
